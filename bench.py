@@ -66,7 +66,15 @@ def parse():
                     help="N > 1, where the resident u16 frames live before the timed region: all on rank 0 (NCCL broadcast per chunk) or 1/N of every "
                          "chunk in each rank's HBM (NCCL all-gather per chunk)")
     ap.add_argument("--emulate-shard", default="", help="R/N: time rank R's shard of an N-GPU run on ONE GPU (no NCCL; development aid)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed steps computed as DIR/<name>.npy (float32 / float64; arrays over "
+                         "the size cap as a fixed seeded sample), to compare two builds output for output (single GPU only)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.emulate_shard):
+        ap.error("--dump-outputs needs the GPU arm without --emulate-shard")
+    return args
 
 
 def metric_name(res):
@@ -177,6 +185,23 @@ def config_dict(args, F, W, H, res, vl, trunc):
             "volume_rule": "dense: every voxel of the box follows Open3D's UniformTSDFVolume::Integrate rule (north_star); the ScalableTSDFVolume "
                            "rule the reference's TSDF() applies (32^3 unit activation, RGB8) is measured beside it as reference_literal",
             "l2": f"inputs larger than L2 ({F * W * H * 2 / 1e9:.2f} GB u16 depth + {res ** 3 * 8 / 1e9:.2f} GB volume per step vs 126 MB)"}
+
+
+# --dump-outputs: at most 2 x 8 MiB of voxels + 12 + 24 + 8 MiB of rows = 60 MiB in all
+DUMP_VOXELS = 1 << 21
+DUMP_ROWS = 1 << 20
+
+
+def dump_sample(n, cap):
+    """indices of a fixed seeded sample of `cap` out of n items (sorted), or None when all n fit"""
+    if n <= cap:
+        return None
+    return np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+
+
+def dump_rows(a, cap=DUMP_ROWS):
+    sel = dump_sample(len(a), cap)
+    return a if sel is None else a[sel]
 
 
 def host_threads():
@@ -323,6 +348,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single-GPU run")
     _lib.require_cuda()
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -429,6 +456,9 @@ def main():
         dist.broadcast(n_settle, 0)          # every rank must run the same number of (collective) steps
     for _ in range(int(n_settle.item())):
         step(depth_u16)
+    # the number of settle steps follows the clock: start the warm-up from an empty volume so that what the timed
+    # steps leave in it depends on --warmup and --steps alone (the work of a step does not depend on the volume)
+    vol.reset()
     for _ in range(args.warmup):
         step(depth_u16)
     vol.profile(True)
@@ -447,6 +477,14 @@ def main():
     stage_ms, k_launches = vol.profile_read_stages()
     k_ms = stage_ms["brick_integrate"]
     vol.profile(False)
+    dumps = {}
+    if args.dump_outputs:
+        # the resident volume after the last timed step, at the same seeded voxel sample in both grids
+        t, w = vol.export_dense()
+        sel = dump_sample(t.numel(), DUMP_VOXELS)
+        sel = slice(None) if sel is None else torch.from_numpy(sel).to(dev)
+        dumps["tsdf"], dumps["weight"] = t.view(-1)[sel].cpu().numpy(), w.view(-1)[sel].cpu().numpy()
+        del t, w, sel
     fps = args.steps * F / (ms_total / 1e3)
     # per-rank timeline of one step (CUDA events inside the library), gathered on rank 0
     steps_prof = max(1, min(args.steps, k_launches // max(len(chunks), 1)))
@@ -515,6 +553,12 @@ def main():
         if mesh is not None:
             nv, nt = int(mesh.vertices.shape[0]), int(mesh.triangles.shape[0])
         mesh_info = {"mc_vertices": nv, "mc_triangles": nt}
+        if args.dump_outputs:
+            # what the last e2e step handed back in host memory
+            dumps["update_counts"] = dump_rows(host_counts.numpy().astype(np.float64))
+            if mesh is not None:
+                dumps["mesh_vertices"] = dump_rows(host_mesh["v"][:nv].numpy())
+                dumps["mesh_triangles"] = dump_rows(host_mesh["t"][:nt].numpy().astype(np.float64))
         e2e = {"value": fps_e2e, "unit": UNIT, "h2d_bytes_per_step": F * H * W * 2 + F * 128, "d2h_bytes_per_step": F * 8 * world + nv * 12 + nt * 12,
                "ms_per_step": ms_e2e / args.steps,
                "includes": "H2D of the u16 frames, a4 + K3 over all frames, " + ("no mesh (--no-mc)" if args.no_mc else
@@ -535,6 +579,11 @@ def main():
             mesh_info["extract_mesh_phase_ms_max_over_ranks"] = {k: max(x[k] for x in allx) for k in mine_x}
             log(f"multi-GPU extraction phases (ms, max over ranks, synchronised between phases): {json.dumps({k: round(v, 2) for k, v in mesh_info['extract_mesh_phase_ms_max_over_ranks'].items()})}")
     clocks = sampler.stop() if sampler else None   # samples inside both timed regions (resident + e2e)
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumps.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
+        log(f"outputs written to {args.dump_outputs}: " + ", ".join(f"{k} {a.dtype}{list(a.shape)}" for k, a in dumps.items()))
 
     # ---- N > 1: the gathered mesh of one clean pass must equal the single-GPU mesh
     parity = {}

@@ -6,6 +6,8 @@ import os
 import sys
 from contextlib import redirect_stdout
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -48,6 +50,17 @@ def test_reference_arm_is_silent_on_other_ranks(monkeypatch):
     with redirect_stdout(buf):
         bench.main()
     assert buf.getvalue() == ""
+
+
+def test_steps_and_dump_outputs_arguments_are_checked(monkeypatch):
+    bench = _bench()
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"], ["--emulate-shard", "0/2", "--dump-outputs", "out"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", *argv])
+        with pytest.raises(SystemExit):
+            bench.parse()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "7", "--dump-outputs", "out"])
+    args = bench.parse()
+    assert args.steps == 7 and args.dump_outputs == "out"
 
 
 def test_workload_table_covers_the_baseline_configs():
