@@ -151,3 +151,21 @@ struct bslam_volume {
     double prof_ms_accum[kProfStages];
     long long prof_launches_accum;
 };
+
+namespace bslam {
+
+// Workspace of the VoxelBlockGrid integrator (bslam_vbg.cu), also read by its ray cast (bslam_raycast.cu): a 256-byte
+// header {u64 ray points seen, u64 ray points outside the box, i32 index of the last frame of the last launch}, the
+// per-block frame masks of the last launch, then the cumulative allocation bitmap (bit b: block b was activated by a
+// frame integrated so far).  Blocks are numbered b = (xb * nby + yb) * nbz + zb.
+constexpr int kVbgBlock = 16;
+constexpr int kVbgMaxFrames = 64;
+constexpr int kVbgMaskWords = kVbgMaxFrames / 32;
+constexpr size_t kVbgLastFrameOffset = 16;
+constexpr size_t kVbgMasksOffset = 256;
+inline size_t vbg_alloc_offset(size_t n_blocks) { return kVbgMasksOffset + n_blocks * kVbgMaskWords * 4; }
+
+// block index of the box corner on the world block grid (origin = b0 * 16 * voxel); BSLAM_E_ARG when the origin is off it
+int vbg_block_origin(const bslam_volume *vol, int b0[3]);
+
+} // namespace bslam

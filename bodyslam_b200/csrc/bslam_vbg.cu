@@ -20,9 +20,6 @@
 
 namespace bslam {
 
-constexpr int kVbgBlock = 16;
-constexpr int kVbgMaxFrames = 64;
-constexpr int kVbgMaskWords = kVbgMaxFrames / 32;
 constexpr int kVbgTouchStride = 4;
 constexpr int kVbgSteps = 3;
 constexpr int kVbgBitmapWords = 8192;      // shared bitmap of the touch kernel: up to 262 144 blocks (1024^3 voxels)
@@ -42,7 +39,7 @@ struct VbgBatch {
 };
 
 __global__ void __launch_bounds__(256) vbg_touch_kernel(const __grid_constant__ VbgBatch bp, const uint16_t *__restrict__ depth, unsigned int *block_masks,
-                                                        unsigned long long *clip) {
+                                                        unsigned int *alloc_bits, int *last_frame, unsigned long long *clip) {
     __shared__ unsigned int s_bits[kVbgBitmapWords];
     const int f = blockIdx.x;
     const int n_blocks = bp.nb[0] * bp.nb[1] * bp.nb[2];
@@ -90,8 +87,10 @@ __global__ void __launch_bounds__(256) vbg_touch_kernel(const __grid_constant__ 
         atomicAdd(clip + 0, (unsigned long long)n_seen);
         if (n_out) atomicAdd(clip + 1, (unsigned long long)n_out);
     }
+    if (threadIdx.x == 0 && f == bp.F - 1) *last_frame = f;
     for (int i = threadIdx.x; i < n_words; i += blockDim.x) {
         unsigned int m = s_bits[i];
+        if (m) atomicOr(&alloc_bits[i], m);
         while (m) {
             const int b = 32 * i + __ffs(m) - 1;
             m &= m - 1;
@@ -169,6 +168,17 @@ __global__ void __launch_bounds__(256) vbg_integrate_kernel(const VolView v, con
     }
 }
 
+int vbg_block_origin(const bslam_volume *vol, int b0[3]) {
+    const double o[3] = {vol->v.ox, vol->v.oy, vol->v.oz};
+    const double bs = vol->voxel_length_d * kVbgBlock;
+    for (int r = 0; r < 3; ++r) {
+        const double k = nearbyint(o[r] / bs);
+        BSLAM_CHECK_ARG(fabs(k * bs - o[r]) <= 1e-9 * fmax(1.0, fabs(o[r])), "origin[%d] = %.12g is not a multiple of the block length %.12g", r, o[r], bs);
+        b0[r] = (int)k;
+    }
+    return BSLAM_OK;
+}
+
 } // namespace bslam
 
 using namespace bslam;
@@ -177,8 +187,9 @@ extern "C" {
 
 size_t bslam_vbg_workspace_bytes(int nx, int ny, int nz) {
     const size_t nb = (size_t)((nx + 15) / 16) * ((ny + 15) / 16) * ((nz + 15) / 16);
-    return nb * kVbgMaskWords * 4 + 256;
+    return vbg_alloc_offset(nb) + (nb + 31) / 32 * 4;
 }
+
 
 int bslam_vbg_integrate(bslam_volume *vol, const uint16_t *d_depth_u16, const uint8_t *d_rgb, int F, int H, int W, const double *h_K,
                         const double *h_poses, const double *h_depth_max, float depth_scale, float trunc_voxel_multiplier,
@@ -199,17 +210,13 @@ int bslam_vbg_integrate(bslam_volume *vol, const uint16_t *d_depth_u16, const ui
     bp.voxel_size = v.vl;
     bp.trunc = v.vl * trunc_voxel_multiplier;
     bp.block_size = v.vl * (float)kVbgBlock;
-    const double o[3] = {v.ox, v.oy, v.oz};
-    const double bs = vol->voxel_length_d * kVbgBlock;
-    for (int r = 0; r < 3; ++r) {
-        const double k = nearbyint(o[r] / bs);
-        BSLAM_CHECK_ARG(fabs(k * bs - o[r]) <= 1e-9 * fmax(1.0, fabs(o[r])), "bslam_vbg_integrate: origin[%d] = %.12g is not a multiple of the block length %.12g", r, o[r], bs);
-        bp.b0[r] = (int)k;
-    }
+    if (vbg_block_origin(vol, bp.b0) != BSLAM_OK) return BSLAM_E_ARG;
     bp.nb[0] = (v.nx + 15) / 16; bp.nb[1] = (v.ny + 15) / 16; bp.nb[2] = (v.nz + 15) / 16;
     const int n_blocks = bp.nb[0] * bp.nb[1] * bp.nb[2];
     BSLAM_CHECK_ARG((n_blocks + 31) / 32 <= kVbgBitmapWords, "bslam_vbg_integrate: too many blocks (%d)", n_blocks);
-    unsigned int *masks = (unsigned int *)((char *)d_workspace + 256);
+    unsigned int *masks = (unsigned int *)((char *)d_workspace + kVbgMasksOffset);
+    unsigned int *alloc_bits = (unsigned int *)((char *)d_workspace + vbg_alloc_offset(n_blocks));
+    int *last_frame = (int *)((char *)d_workspace + kVbgLastFrameOffset);
     unsigned long long *clip = (unsigned long long *)d_workspace;
     const int64_t n_pix = (int64_t)W * H;
     for (int f0 = 0; f0 < F; f0 += kVbgMaxFrames) {
@@ -232,7 +239,7 @@ int bslam_vbg_integrate(bslam_volume *vol, const uint16_t *d_depth_u16, const ui
             fp.depth_max = (float)h_depth_max[f0 + f];
         }
         BSLAM_CUDA(cudaMemsetAsync(masks, 0, (size_t)n_blocks * kVbgMaskWords * 4, st));
-        vbg_touch_kernel<<<nf, 256, 0, st>>>(bp, d_depth_u16 + f0 * n_pix, masks, clip);
+        vbg_touch_kernel<<<nf, 256, 0, st>>>(bp, d_depth_u16 + f0 * n_pix, masks, alloc_bits, last_frame, clip);
         BSLAM_LAUNCH_CHECK();
         unsigned long long *cnt = d_update_counts ? d_update_counts + f0 : nullptr;
         if (vol->with_color)

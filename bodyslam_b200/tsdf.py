@@ -6,6 +6,8 @@ Where the reference wraps Open3D's CPU `ScalableTSDFVolume`, `.tsdf` here is a
 `DenseTSDFVolume`: the dense N^3 equivalent (Open3D UniformTSDFVolume semantics) living
 brick-ordered in B200 HBM and driven by the hand-written kernels in csrc/.  Extra, non-breaking
 keyword arguments choose the box (`resolution`, `origin`), colour integration and the device.
+Both volumes can be ray cast: `DenseTSDFVolume.raycast` and `MAP.synthesize_model_frame` render depth, vertex,
+normal and colour maps of the map from a pose (csrc/bslam_raycast.cu).
 """
 from __future__ import annotations
 
@@ -493,6 +495,38 @@ class DenseTSDFVolume:
             _lib.check(self._L.bslam_tsdf_export_plane(self._h, int(z), _lib.ptr(p), _lib.stream_ptr(self.device)))
         return p
 
+    # ------------------------------------------------------------------ ray casting
+    def _raycast_outputs(self, F, H, W, normals, colors):
+        torch = _lib.require_cuda()
+        dev = self.device
+        out = {"depth": torch.empty((F, H, W), dtype=torch.float32, device=dev),
+               "vertex": torch.empty((F, H, W, 3), dtype=torch.float32, device=dev)}
+        if normals:
+            out["normal"] = torch.empty((F, H, W, 3), dtype=torch.float32, device=dev)
+        if colors:
+            out["color"] = torch.empty((F, H, W, 3), dtype=torch.float32, device=dev)
+        return out
+
+    def raycast(self, intrinsic, extrinsics, depth_min: float = 0.0, depth_max: float = 3.0, depth_scale: float = 1.0,
+                weight_threshold: float = 0.0, normals: bool = True, colors=None):
+        """Render the volume from F poses: one ray per pixel marches the TSDF to its first zero crossing of valid voxels
+        (weight >= weight_threshold; != 0 when it is 0) between depth_min and depth_max (metres along the camera z).
+        extrinsics: [F,4,4] or one 4x4 world -> camera (f64).  colors: None = when the volume has colour.
+        -> dict of CUDA f32 tensors: depth [F,H,W] (z * depth_scale), vertex [F,H,W,3] (camera frame), normal
+        [F,H,W,3] (camera frame, unit) when `normals`, color [F,H,W,3] in [0, 1] when colours are asked for; pixels
+        whose ray hits nothing are 0.  The volume is not changed (single-box volumes, dims multiples of 8)."""
+        torch = _lib.require_cuda()
+        W, H, fx, fy, cx, cy = intrinsic_params(intrinsic)
+        E = np.ascontiguousarray(np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 16))
+        colors = self.color if colors is None else bool(colors)
+        out = self._raycast_outputs(E.shape[0], H, W, normals, colors)
+        K = np.array([fx, fy, cx, cy], dtype=np.float64)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.bslam_tsdf_raycast(self._h, E.shape[0], H, W, _lib.ptr(K), _lib.ptr(E), float(depth_scale), float(depth_min),
+                                                  float(depth_max), float(weight_threshold), _lib.ptr(out["depth"]), _lib.ptr(out["vertex"]),
+                                                  _lib.ptr(out.get("normal")), _lib.ptr(out.get("color")), _lib.stream_ptr(self.device)))
+        return out
+
     # ------------------------------------------------------------------ extraction
     def mc_count(self, halo_lo=None, halo_hi=None):
         """first phase of the marching cubes: (vertices, triangles) this box will emit (synchronises)"""
@@ -704,8 +738,9 @@ class MAP:
     `trunc_voxel_multiplier`).  Same constructor and methods; the blocks live in a bounded dense box
     (extra kwargs `resolution`, `origin`, `color`) instead of Open3D's hash map of `block_count` blocks
     (`block_count` is accepted and ignored; ray points that leave the box are counted, see `clip_stats`).
-    `synthesize_model_frame` (ray casting into `raycast_frame`, whose result the reference discards) is not
-    provided.  Extraction follows the tensor pipeline's defaults: weight threshold 3, vertices on voxel corners.
+    Extraction follows the tensor pipeline's defaults: weight threshold 3, vertices on voxel corners.
+    `synthesize_model_frame` ray casts the map from the pose of the last integrated frame (Open3D's
+    `Model.synthesize_model_frame`); `integrate` does not call it (the reference discards its result).
     """
 
     BLOCK = 16
@@ -735,6 +770,8 @@ class MAP:
         _lib.check(self.model._L.bslam_tsdf_set_extract_flavour(self.model._h, float(weight_threshold), 0.0))
         self._ws = torch.zeros(self.model._L.bslam_vbg_workspace_bytes(*res), dtype=torch.uint8, device=dev)
         self.poses = {}
+        self._last_pose, self._frame_id = None, -1
+        self._range_ws = None
 
     def integrate_batch(self, depth_u16, color, poses, depth_max, update_counts=None):
         """F frames in order: depth_u16 [F,H,W] uint16 (raw, divided by depth_scale in the kernel), color
@@ -765,6 +802,8 @@ class MAP:
                                                   _lib.ptr(dm), self.depth_scale, self.trunc_voxel_multiplier, _lib.ptr(self._ws),
                                                   _lib.ptr(update_counts), _lib.stream_ptr(vol.device)))
         vol.frames_integrated += F
+        if F:
+            self._last_pose, self._frame_id = P[-1].copy(), vol.frames_integrated - 1
 
     def integrate(self, curr_rgbd, i, curr_global_pose):
         """reference signature (tsdf.py:71): `curr_rgbd` is an `RGBD` (uses `.o3d_t_depth`, `.o3d_t_color`,
@@ -772,6 +811,48 @@ class MAP:
         pose = np.asarray(to_numpy(curr_global_pose), dtype=np.float64).reshape(4, 4)
         self.poses[int(i)] = pose
         self.integrate_batch(curr_rgbd.o3d_t_depth, curr_rgbd.o3d_t_color if self.model.color else None, pose[None], curr_rgbd.depth_max)
+        self._frame_id = int(i)
+
+    def synthesize_model_frame(self, depth_min: float = 0.1, depth_max: float = 3.0, enable_color: bool = True, weight_threshold: float = -1.0):
+        """Open3D `Model.synthesize_model_frame`: ray cast the map at width x height from the pose of the last integrated
+        frame, over the ray ranges of the blocks that frame activated.  weight_threshold < 0: min(frame_id, 3), frame_id =
+        the last `i` given to `integrate` (as recalled from Open3D's SynthesizeModelFrame).  -> dict of CUDA f32 tensors
+        depth [1,H,W] (raw units: z * depth_scale), vertex / normal [1,H,W,3] (camera frame), color [1,H,W,3] in [0, 1]
+        (colour maps and enable_color only); pixels whose ray hits nothing are 0."""
+        torch = _lib.require_cuda()
+        if self._last_pose is None:
+            raise RuntimeError("[MAP::SynthesizeModelFrame] nothing integrated yet")
+        vol = self.model
+        if weight_threshold < 0:
+            weight_threshold = min(float(self._frame_id), 3.0)
+        H, W = self.height, self.width
+        out = vol._raycast_outputs(1, H, W, True, enable_color and vol.color)
+        nbytes = vol._L.bslam_vbg_raycast_workspace_bytes(H, W)
+        if self._range_ws is None or self._range_ws.numel() < nbytes:
+            self._range_ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=vol.device)
+        P = np.ascontiguousarray(self._last_pose.reshape(16))
+        with torch.cuda.device(vol.device):
+            _lib.check(vol._L.bslam_vbg_raycast(vol._h, _lib.ptr(self._ws), H, W, _lib.ptr(self._K), _lib.ptr(P), self.depth_scale, float(depth_min),
+                                                float(depth_max), float(weight_threshold), self.trunc_voxel_multiplier, _lib.ptr(out["depth"]),
+                                                _lib.ptr(out["vertex"]), _lib.ptr(out["normal"]), _lib.ptr(out.get("color")), _lib.ptr(self._range_ws),
+                                                _lib.stream_ptr(vol.device)))
+        return out
+
+    def allocated_blocks(self, last_frame: bool = False):
+        """bool CUDA tensor [nbx, nby, nbz] of the 16^3 blocks of the box: activated by any frame integrated so far (the
+        VoxelBlockGrid's allocated blocks), or with `last_frame` by the last integrated frame only (synchronises)."""
+        torch = _lib.require_cuda()
+        vol = self.model
+        nb = [n // self.BLOCK for n in (vol.nx, vol.ny, vol.nz)]
+        n = nb[0] * nb[1] * nb[2]
+        bit = torch.arange(32, dtype=torch.int32, device=vol.device)
+        if last_frame:
+            f = int(self._ws[16:20].view(torch.int32).item())
+            masks = self._ws[256:256 + n * 8].view(torch.int32).view(n, 2)[:, f >> 5]
+            return ((masks >> (f & 31)) & 1).bool().view(nb)
+        off = 256 + n * 8
+        words = self._ws[off:off + (n + 31) // 32 * 4].view(torch.int32)
+        return ((words[:, None] >> bit) & 1).bool().reshape(-1)[:n].view(nb)
 
     def clip_stats(self):
         """ray points of the block activation seen / outside the bounded box (the reference's hash map is unbounded)"""

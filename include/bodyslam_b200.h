@@ -331,13 +331,40 @@ BSLAM_API int bslam_mesh_merge(int n_slabs, const int64_t *h_nv, const int64_t *
  * camera->world (T_frame_to_model), h_depth_max [F] f64 (`curr_rgbd.depth_max`).  d_workspace:
  * bslam_vbg_workspace_bytes() bytes, ZEROED by the caller once; its first 16 bytes accumulate {ray points
  * seen, ray points outside the box} (bslam_vbg_stats; the reference's hash map is unbounded).
- * `synthesize_model_frame` (ray casting, whose result MAP discards) is not provided. */
+ * The workspace also keeps, across calls, the blocks activated by any frame so far (the VoxelBlockGrid's allocated
+ * blocks) and the blocks the last integrated frame activated; bslam_vbg_raycast reads both. */
 BSLAM_API size_t bslam_vbg_workspace_bytes(int nx, int ny, int nz);
 BSLAM_API int bslam_vbg_integrate(bslam_volume *vol, const uint16_t *d_depth_u16, const uint8_t *d_rgb, int F, int H, int W,
                                   const double *h_K, const double *h_poses, const double *h_depth_max, float depth_scale,
                                   float trunc_voxel_multiplier, void *d_workspace, unsigned long long *d_update_counts,
                                   bslam_stream_t stream);
 BSLAM_API int bslam_vbg_stats(const void *d_workspace, unsigned long long *h_stat2, bslam_stream_t stream);
+/* ------------------------------------------------------------------ ray casting (row f4)
+ * Rendered depth, vertex, normal and colour maps of the volume from a pose: Open3D's tensor RayCast (the semantics,
+ * and where they deliberately differ from Open3D, are written down in its CPU reference, tests/raycast_ref.c).  One ray
+ * per integer pixel; a ray that finds no zero crossing of valid voxels (weight >= weight_threshold, or != 0 when it
+ * is 0) writes zeros.  depth = z in the camera frame * depth_scale; vertex and normal are in the camera frame; colour
+ * in [0, 1].  Outputs: d_depth [F][H][W] f32 (required), d_vertex, d_normal, d_color [F][H][W][3] f32 (each optional,
+ * NULL = not produced; a colour map needs a colour volume).  The volume is read only.
+ *
+ * bslam_tsdf_raycast: legacy flavour on a DenseTSDFVolume box (dense, unit-activation or unit-arithmetic mode; dims
+ * multiples of 8; not z-sharded or z-interleaved): 8^3 bricks relative to the box origin, brick flag bit 0 as the
+ * allocation, voxel-centre trilinear interpolation, sdf_trunc of the volume, ray range [depth_min, depth_max].
+ * h_extrinsics [F][16] f64 world -> camera; any F (launched 64 frames at a time). */
+BSLAM_API int bslam_tsdf_raycast(bslam_volume *vol, int F, int H, int W, const double *h_K, const double *h_extrinsics, float depth_scale,
+                                 float depth_min, float depth_max, float weight_threshold, float *d_depth, float *d_vertex, float *d_normal,
+                                 float *d_color, bslam_stream_t stream);
+/* bslam_vbg_raycast: tensor flavour (`MAP.synthesize_model_frame`) on a volume integrated by bslam_vbg_integrate with
+ * the workspace d_vbg_workspace: 16^3 blocks on the world block grid, allocated = activated by any frame so far,
+ * voxel-corner trilinear interpolation, sdf_trunc = trunc_voxel_multiplier * voxel_size, ray range from Open3D's
+ * EstimateRange (down factor 8) over the blocks the last integrated frame activated.  h_pose [16] f64 camera -> world;
+ * H, W >= 8.  d_range_workspace: bslam_vbg_raycast_workspace_bytes(H, W) bytes of device scratch (the range map). */
+BSLAM_API size_t bslam_vbg_raycast_workspace_bytes(int H, int W);
+BSLAM_API int bslam_vbg_raycast(bslam_volume *vol, const void *d_vbg_workspace, int H, int W, const double *h_K, const double *h_pose,
+                                float depth_scale, float depth_min, float depth_max, float weight_threshold, float trunc_voxel_multiplier,
+                                float *d_depth, float *d_vertex, float *d_normal, float *d_color, void *d_range_workspace,
+                                bslam_stream_t stream);
+
 /* Surface-extraction flavour of bslam_mc_* / bslam_points_*: a voxel is valid when weight >= weight_threshold
  * (0 = Open3D's legacy `weight != 0`; the tensor pipeline's extract_triangle_mesh / extract_point_cloud default is 3)
  * and vertices sit at (index + vertex_offset) * voxel_length (legacy 0.5 = voxel centres; tensor pipeline 0). */
