@@ -287,11 +287,12 @@ static void rc_common(RcBatch &bp, const VolView &v, int H, int W, const double 
 
 using namespace bslam;
 
-#define RC_CHECK_COMMON(name)                                                                                                          \
+// n_frames == 0: the outputs are empty, so their pointers may be NULL (an empty tensor's data pointer)
+#define RC_CHECK_COMMON(name, n_frames)                                                                                                \
     BSLAM_CHECK_ARG(H > 0 && W > 0, "[" name "] Unsupported image format. (H=%d W=%d)", H, W);                                          \
     BSLAM_CHECK_ARG(depth_scale > 0.f && depth_min >= 0.f && isfinite(depth_min) && isfinite(depth_max) && weight_threshold >= 0.f,     \
                     name ": depth_scale must be > 0, depth_min >= 0, depth_max finite and weight_threshold >= 0");                     \
-    BSLAM_CHECK_ARG(vol && h_K && d_depth, name ": NULL argument");                                                                  \
+    BSLAM_CHECK_ARG(vol && h_K && (d_depth || (n_frames) == 0), name ": NULL argument");                                            \
     BSLAM_CHECK_ARG(!(d_color && !vol->with_color), "[" name "] a colour map needs a colour volume");                                 \
     BSLAM_CHECK_ARG(vol->v.zs == 1 && vol->v.gz0 == 0 && (vol->z_total == 0 || vol->z_total == vol->v.nz),                            \
                     name ": single-box volumes only (no z-sharded or z-interleaved boxes)")
@@ -302,8 +303,8 @@ int bslam_tsdf_raycast(bslam_volume *vol, int F, int H, int W, const double *h_K
                        float depth_min, float depth_max, float weight_threshold, float *d_depth, float *d_vertex, float *d_normal,
                        float *d_color, bslam_stream_t stream) {
     BSLAM_CHECK_ARG(F >= 0, "[bslam_tsdf_raycast] Unsupported image format. (F=%d)", F);
-    RC_CHECK_COMMON("bslam_tsdf_raycast");
-    BSLAM_CHECK_ARG(h_extrinsics, "bslam_tsdf_raycast: NULL argument");
+    RC_CHECK_COMMON("bslam_tsdf_raycast", F);
+    BSLAM_CHECK_ARG(h_extrinsics || F == 0, "bslam_tsdf_raycast: NULL argument");
     const VolView &v = vol->v;
     BSLAM_CHECK_ARG(v.nx % kBrick == 0 && v.ny % kBrick == 0 && v.nz % kBrick == 0, "bslam_tsdf_raycast: the box must consist of whole %d^3 bricks", kBrick);
     if (F == 0) return BSLAM_OK;
@@ -338,7 +339,7 @@ int bslam_vbg_raycast(bslam_volume *vol, const void *d_vbg_workspace, int H, int
                       float depth_min, float depth_max, float weight_threshold, float trunc_voxel_multiplier, float *d_depth, float *d_vertex,
                       float *d_normal, float *d_color, void *d_range_workspace, bslam_stream_t stream) {
     BSLAM_CHECK_ARG(H >= kRcDown && W >= kRcDown, "[bslam_vbg_raycast] Unsupported image format. (H=%d W=%d; at least %d x %d)", H, W, kRcDown, kRcDown);
-    RC_CHECK_COMMON("bslam_vbg_raycast");
+    RC_CHECK_COMMON("bslam_vbg_raycast", 1);
     BSLAM_CHECK_ARG(d_vbg_workspace && h_pose && d_range_workspace, "bslam_vbg_raycast: NULL argument");
     BSLAM_CHECK_ARG(trunc_voxel_multiplier > 0.f, "bslam_vbg_raycast: trunc_voxel_multiplier must be > 0");
     const VolView &v = vol->v;
