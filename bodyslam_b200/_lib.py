@@ -57,8 +57,9 @@ _SIGNATURES = {
     "bslam_tsdf_export": (C.c_int, [_p, _p, _p, _p, _p]),
     "bslam_tsdf_import": (C.c_int, [_p, _p, _p, _p, _p]),
     "bslam_tsdf_export_plane": (C.c_int, [_p, C.c_int, _p, _p]),
+    "bslam_tsdf_export_plane_color": (C.c_int, [_p, C.c_int, _p, _p]),
     "bslam_mc_count": (C.c_int, [_p, _p, _p, _p, _p]),
-    "bslam_mc_emit": (C.c_int, [_p, _p, _p, _p, _p, _p, C.c_int64, _p, C.c_int64, _p]),
+    "bslam_mc_emit": (C.c_int, [_p, _p, _p, _p, _p, _p, _p, C.c_int64, _p, C.c_int64, _p]),
     "bslam_mesh_merge_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "bslam_mesh_merge": (C.c_int, [C.c_int, _p, _p, _p, C.c_int, C.c_int, _p, _p, _p, _p, _p]),
     "bslam_vbg_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),

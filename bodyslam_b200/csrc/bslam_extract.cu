@@ -140,8 +140,8 @@ __device__ __forceinline__ BrickClass classify_brick(const VolView &v, const flo
 }
 
 template <bool EMIT>
-__global__ void __launch_bounds__(kBrickVox) mc_brick_kernel(const VolView v, double vld, const float2 *halo_lo, const float2 *halo_hi, McScratch sc,
-                                                              float *vertices, int32_t *keys, float *colors, int64_t cap_v,
+__global__ void __launch_bounds__(kBrickVox) mc_brick_kernel(const VolView v, double vld, const float2 *halo_lo, const float2 *halo_hi,
+                                                              const float *halo_hi_color, McScratch sc, float *vertices, int32_t *keys, float *colors, int64_t cap_v,
                                                               int32_t *tris, int64_t cap_t) {
     __shared__ float s_t[kR * kR * kR];
     __shared__ uint8_t s_ok[kR * kR * kR];
@@ -211,11 +211,13 @@ __global__ void __launch_bounds__(kBrickVox) mc_brick_kernel(const VolView v, do
         if (colors && v.color) {
             const int64_t s0 = voxel_slot(v, X, Y, Z);
             const int X1 = X + (a == 0), Y1 = Y + (a == 1), Z1 = Z + (a == 2);
-            // colour of a voxel on the halo_hi plane is not available: reuse the owner's colour
-            const int64_t s1 = (Z1 < v.nz) ? voxel_slot(v, X1, Y1, Z1) : s0;
+            // the far end of a z-edge from the top plane lies on the halo_hi plane: its colour comes from the slab above
+            const bool hi = Z1 >= v.nz;
+            const int64_t s1 = hi ? 0 : voxel_slot(v, X1, Y1, Z1);
             for (int k = 0; k < 3; ++k) {
                 const double c0 = v.color[(s0 / kBrickVox) * (3 * kBrickVox) + k * kBrickVox + (s0 % kBrickVox)];
-                const double c1 = v.color[(s1 / kBrickVox) * (3 * kBrickVox) + k * kBrickVox + (s1 % kBrickVox)];
+                const double c1 = hi ? halo_hi_color[((int64_t)X1 * v.ny + Y1) * 3 + k]
+                                     : v.color[(s1 / kBrickVox) * (3 * kBrickVox) + k * kBrickVox + (s1 % kBrickVox)];
                 colors[3 * id + k] = (float)(((f1 * c0 + f0 * c1) / (f0 + f1)) / 255.0);
             }
         }
@@ -761,8 +763,8 @@ int bslam_mc_count(bslam_volume *vol, const float *d_halo_lo, const float *d_hal
     const McScratch sc = carve_mc(vol->mc_scratch, (size_t)nb);
     rc = build_candidates(vol, sc, d_halo_hi != nullptr, st);
     if (rc) return rc;
-    mc_brick_kernel<false><<<kExtractGrid, kBrickVox, 0, st>>>(vol->v, vol->voxel_length_d, (const float2 *)d_halo_lo, (const float2 *)d_halo_hi, sc, nullptr, nullptr,
-                                                               nullptr, 0, nullptr, 0);
+    mc_brick_kernel<false><<<kExtractGrid, kBrickVox, 0, st>>>(vol->v, vol->voxel_length_d, (const float2 *)d_halo_lo, (const float2 *)d_halo_hi, nullptr, sc,
+                                                               nullptr, nullptr, nullptr, 0, nullptr, 0);
     BSLAM_LAUNCH_CHECK();
     rc = brick_scan(sc.nvert, sc.ntri, sc.vbase, sc.tbase, nb, sc.totals, sc.scan_ws, st);
     if (rc) return rc;
@@ -774,15 +776,17 @@ int bslam_mc_count(bslam_volume *vol, const float *d_halo_lo, const float *d_hal
     return BSLAM_OK;
 }
 
-int bslam_mc_emit(bslam_volume *vol, const float *d_halo_lo, const float *d_halo_hi, float *d_vertices, int32_t *d_keys, float *d_colors,
-                  int64_t cap_v, int32_t *d_tri, int64_t cap_t, bslam_stream_t stream) {
+int bslam_mc_emit(bslam_volume *vol, const float *d_halo_lo, const float *d_halo_hi, const float *d_halo_hi_color, float *d_vertices,
+                  int32_t *d_keys, float *d_colors, int64_t cap_v, int32_t *d_tri, int64_t cap_t, bslam_stream_t stream) {
     BSLAM_CHECK_ARG(vol && vol->mc_scratch, "bslam_mc_emit: call bslam_mc_count first");
     BSLAM_CHECK_ARG((d_vertices || cap_v == 0) && (d_tri || cap_t == 0), "bslam_mc_emit: NULL output");
+    BSLAM_CHECK_ARG(!(d_colors && vol->v.color && d_halo_hi && !d_halo_hi_color),
+                    "bslam_mc_emit: colours with a halo_hi plane need its colour plane (bslam_tsdf_export_plane_color)");
     BSLAM_DEVICE_GUARD(vol->device);
     const int64_t nb = brick_count(vol->v);
     const McScratch sc = carve_mc(vol->mc_scratch, (size_t)nb);
-    mc_brick_kernel<true><<<kExtractGrid, kBrickVox, 0, (cudaStream_t)stream>>>(vol->v, vol->voxel_length_d, (const float2 *)d_halo_lo, (const float2 *)d_halo_hi, sc,
-                                                                                 d_vertices, d_keys, d_colors, cap_v, d_tri, cap_t);
+    mc_brick_kernel<true><<<kExtractGrid, kBrickVox, 0, (cudaStream_t)stream>>>(vol->v, vol->voxel_length_d, (const float2 *)d_halo_lo, (const float2 *)d_halo_hi,
+                                                                                 d_halo_hi_color, sc, d_vertices, d_keys, d_colors, cap_v, d_tri, cap_t);
     BSLAM_LAUNCH_CHECK();
     return BSLAM_OK;
 }

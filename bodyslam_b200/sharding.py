@@ -123,6 +123,25 @@ def exchange_halo_planes(top_plane, bottom_plane, rank: int, world_size: int, gr
     return halo_lo, halo_hi
 
 
+def exchange_halo_color(bottom_color, rank: int, world_size: int, group=None):
+    """colour half of the halo exchange: every rank sends the colour of its bottom plane to rank-1 and returns
+    halo_hi_color = the colour of rank+1's bottom plane (None on the last rank).  Only the slab below needs it:
+    a vertex on a z-edge from its top plane interpolates towards that plane's colour."""
+    import torch
+    import torch.distributed as dist
+
+    halo_hi_color = torch.empty_like(bottom_color) if rank + 1 < world_size else None
+    ops_ = []
+    if rank + 1 < world_size:
+        ops_.append(dist.P2POp(dist.irecv, halo_hi_color, rank + 1, group))
+    if rank > 0:
+        ops_.append(dist.P2POp(dist.isend, bottom_color, rank - 1, group))
+    if ops_:
+        for w in dist.batch_isend_irecv(ops_):
+            w.wait()
+    return halo_hi_color
+
+
 def _pack_mesh(mesh: TriangleMesh):
     """vertices f32 [V,3] | keys i32 [V,4] | triangles i32 [T,3] | colours f32 [V,3] as ONE int32 buffer"""
     import torch
@@ -542,14 +561,15 @@ class ShardedTSDF:
         v = self.contiguous_slab()
         mark()
         lo, hi = exchange_halo_planes(v.export_plane(v.nz - 1), v.export_plane(0), self.rank, self.world_size, self.group)
+        hi_col = exchange_halo_color(v.export_plane_color(0), self.rank, self.world_size, self.group) if v.color else None
         mark()
-        out = self._gather_slab_meshes(v, lo, hi, profile_mark=mark)
+        out = self._gather_slab_meshes(v, lo, hi, hi_col, profile_mark=mark)
         if profile:
             names = ("reshard_to_slabs", "halo_exchange", "marching_cubes_count", "sizes_allgather", "emit_and_gather", "merge")
             self.last_extract_profile = {n: 1e3 * (b - a) for n, a, b in zip(names, t[:-1], t[1:])}
         return out
 
-    def _gather_slab_meshes(self, v, lo, hi, profile_mark=lambda: None):
+    def _gather_slab_meshes(self, v, lo, hi, hi_col=None, profile_mark=lambda: None):
         """count per slab -> sizes to everybody -> rank 0 allocates the WHOLE mesh once; every slab's marching cubes
         emit straight into its rows (rank 0) or into a send buffer (others) and the pieces are received in place ->
         two small kernels (bslam_mesh_merge) rebase the vertex ids and resolve the cross-slab references."""
@@ -573,7 +593,7 @@ class ShardedTSDF:
             keys = torch.empty((V, 4), dtype=torch.int32, device=dev)
             cols = torch.empty((V, 3), dtype=torch.float32, device=dev) if v.color else None
             tris = torch.empty((T, 3), dtype=torch.int32, device=dev)
-            v.mc_emit(verts, keys, cols, tris, lo, hi)
+            v.mc_emit(verts, keys, cols, tris, lo, hi, hi_col)
             ops_ = [dist.P2POp(dist.isend, t, 0, self.group) for t in (verts, keys, tris, cols) if t is not None and t.numel()]
             if ops_:
                 for w in dist.batch_isend_irecv(ops_):
@@ -593,7 +613,7 @@ class ShardedTSDF:
             for t, b in ((verts, vb), (keys, vb), (tris, tb), (cols, vb)):
                 if t is not None and b[r + 1] > b[r]:
                     ops_.append(dist.P2POp(dist.irecv, t[b[r]:b[r + 1]], r, self.group))
-        v.mc_emit(verts[:V], keys[:V], None if cols is None else cols[:V], tris[:T], lo, hi)
+        v.mc_emit(verts[:V], keys[:V], None if cols is None else cols[:V], tris[:T], lo, hi, hi_col)
         if ops_:
             for w in dist.batch_isend_irecv(ops_):
                 w.wait()

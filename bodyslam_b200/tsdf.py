@@ -495,6 +495,14 @@ class DenseTSDFVolume:
             _lib.check(self._L.bslam_tsdf_export_plane(self._h, int(z), _lib.ptr(p), _lib.stream_ptr(self.device)))
         return p
 
+    def export_plane_color(self, z: int):
+        """colour of local plane z as a [nx, ny, 3] f32 CUDA tensor in [0, 255] (colour halo of the slab below)."""
+        torch = _lib.require_cuda()
+        p = torch.empty((self.nx, self.ny, 3), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.bslam_tsdf_export_plane_color(self._h, int(z), _lib.ptr(p), _lib.stream_ptr(self.device)))
+        return p
+
     # ------------------------------------------------------------------ ray casting
     def _raycast_outputs(self, F, H, W, normals, colors):
         torch = _lib.require_cuda()
@@ -536,9 +544,10 @@ class DenseTSDFVolume:
             _lib.check(self._L.bslam_mc_count(self._h, _lib.ptr(halo_lo), _lib.ptr(halo_hi), _lib.ptr(cnt), _lib.stream_ptr(self.device)))
         return int(cnt[0]), int(cnt[1])
 
-    def mc_emit(self, verts, keys, cols, tris, halo_lo=None, halo_hi=None):
+    def mc_emit(self, verts, keys, cols, tris, halo_lo=None, halo_hi=None, halo_hi_color=None):
         """second phase: write this box's mesh into caller tensors (slices of a gathered mesh, for example):
-        verts [V,3] f32, keys [V,4] i32, cols [V,3] f32 | None, tris [T,3] i32 -- all contiguous CUDA tensors"""
+        verts [V,3] f32, keys [V,4] i32, cols [V,3] f32 | None, tris [T,3] i32 -- all contiguous CUDA tensors.
+        halo_hi_color: `export_plane_color(0)` of the slab above; needed for colours together with halo_hi."""
         torch = _lib.require_cuda()
         V, T = int(verts.shape[0]), int(tris.shape[0])
         if not (V or T):
@@ -547,18 +556,20 @@ class DenseTSDFVolume:
             if t is not None and not t.is_contiguous():
                 raise RuntimeError("mc_emit: output tensors must be contiguous")
         with torch.cuda.device(self.device):
-            _lib.check(self._L.bslam_mc_emit(self._h, _lib.ptr(halo_lo), _lib.ptr(halo_hi), _lib.ptr(verts), _lib.ptr(keys),
-                                             _lib.ptr(cols) if self.color else None, V, _lib.ptr(tris), T, _lib.stream_ptr(self.device)))
+            _lib.check(self._L.bslam_mc_emit(self._h, _lib.ptr(halo_lo), _lib.ptr(halo_hi), _lib.ptr(halo_hi_color), _lib.ptr(verts),
+                                             _lib.ptr(keys), _lib.ptr(cols) if self.color else None, V, _lib.ptr(tris), T,
+                                             _lib.stream_ptr(self.device)))
 
-    def extract_triangle_mesh(self, halo_lo=None, halo_hi=None) -> TriangleMesh:
-        """Open3D `extract_triangle_mesh()` (tsdf.py:43) -- compacted marching cubes on the GPU."""
+    def extract_triangle_mesh(self, halo_lo=None, halo_hi=None, halo_hi_color=None) -> TriangleMesh:
+        """Open3D `extract_triangle_mesh()` (tsdf.py:43) -- compacted marching cubes on the GPU.  Slab of a z-sharded
+        volume: halo_lo / halo_hi are the neighbours' planes (`export_plane`), halo_hi_color the upper one's colour."""
         torch = _lib.require_cuda()
         V, T = self.mc_count(halo_lo, halo_hi)
         verts = torch.empty((V, 3), dtype=torch.float32, device=self.device)
         keys = torch.empty((V, 4), dtype=torch.int32, device=self.device)
         cols = torch.empty((V, 3), dtype=torch.float32, device=self.device) if self.color else None
         tris = torch.empty((T, 3), dtype=torch.int32, device=self.device)
-        self.mc_emit(verts, keys, cols, tris, halo_lo, halo_hi)
+        self.mc_emit(verts, keys, cols, tris, halo_lo, halo_hi, halo_hi_color)
         return TriangleMesh(verts, tris, cols, keys)
 
     def set_incremental_points(self, enable: bool = True, normals: bool = True):

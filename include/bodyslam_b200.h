@@ -287,6 +287,9 @@ BSLAM_API int bslam_tsdf_import(bslam_volume *vol, const float *d_tsdf, const fl
 /* {tsdf,weight} of local plane z as [nx][ny] float2 (halo exchange between z-slabs) */
 BSLAM_API int bslam_tsdf_export_plane(const bslam_volume *vol, int z, float *d_plane_f2,
                                       bslam_stream_t stream);
+/* colour of local plane z as [nx][ny][3] f32 in [0,255] (colour volumes): the d_halo_hi_color of the slab below */
+BSLAM_API int bslam_tsdf_export_plane_color(const bslam_volume *vol, int z, float *d_plane_rgb,
+                                            bslam_stream_t stream);
 
 /* ------------------------------------------------------------------ surface extraction (K4)
  * Replaces `TSDF.extract_mesh()` N/3DM/tsdf.py:42-43 (Open3D extract_triangle_mesh):
@@ -302,11 +305,14 @@ BSLAM_API int bslam_tsdf_export_plane(const bslam_volume *vol, int z, float *d_p
  * callers canonicalise.  Vertex ids in d_tri are local to this box unless the edge is owned
  * by plane z = nz, in which case the id is -(1 + (x*ny + y)*4 + axis) (resolved on gather).
  * d_vertices [cap_v][3] f32 world; d_colors optional [cap_v][3] f32 in [0,1] (colour volumes);
- * d_tri [cap_t][3] i32.  Rows beyond capacity are not written. */
+ * d_tri [cap_t][3] i32.  Rows beyond capacity are not written.
+ * d_halo_hi_color: [nx][ny][3] f32 colour of the d_halo_hi plane (bslam_tsdf_export_plane_color of the slab above).
+ * A vertex on a z-edge from this slab's top plane interpolates its colour with it, as the single-box mesh does.
+ * Required when d_halo_hi, d_colors and a colour volume are given; ignored otherwise (NULL). */
 BSLAM_API int bslam_mc_count(bslam_volume *vol, const float *d_halo_lo, const float *d_halo_hi,
                              int64_t *h_counts /* [2]: V, T */, bslam_stream_t stream);
 BSLAM_API int bslam_mc_emit(bslam_volume *vol, const float *d_halo_lo, const float *d_halo_hi,
-                            float *d_vertices, int32_t *d_keys, float *d_colors, int64_t cap_v,
+                            const float *d_halo_hi_color, float *d_vertices, int32_t *d_keys, float *d_colors, int64_t cap_v,
                             int32_t *d_tri, int64_t cap_t, bslam_stream_t stream);
 
 /* Gather side of the z-slab meshes ("per-slab meshes concatenated on gather", north_star): the slabs' d_keys [V][4]
@@ -366,8 +372,9 @@ BSLAM_API int bslam_vbg_raycast(bslam_volume *vol, const void *d_vbg_workspace, 
                                 bslam_stream_t stream);
 
 /* Surface-extraction flavour of bslam_mc_* / bslam_points_*: a voxel is valid when weight >= weight_threshold
- * (0 = Open3D's legacy `weight != 0`; the tensor pipeline's extract_triangle_mesh / extract_point_cloud default is 3)
- * and vertices sit at (index + vertex_offset) * voxel_length (legacy 0.5 = voxel centres; tensor pipeline 0). */
+ * (0 = weight > 0, Open3D's legacy `weight != 0` for every weight an integrator writes: they differ only for negative
+ * or NaN weights, which count as invalid here; the tensor pipeline's extract_triangle_mesh / extract_point_cloud default
+ * is 3) and vertices sit at (index + vertex_offset) * voxel_length (legacy 0.5 = voxel centres; tensor pipeline 0). */
 BSLAM_API int bslam_tsdf_set_extract_flavour(bslam_volume *vol, float weight_threshold, double vertex_offset);
 
 /* Replaces `TSDF.extract_pcd()` N/3DM/tsdf.py:39-40 (Open3D extract_point_cloud): interior

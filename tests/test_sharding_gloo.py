@@ -11,7 +11,7 @@ import torch.multiprocessing as mp
 
 import oracle
 from bodyslam_b200.geometry import TriangleMesh
-from bodyslam_b200.sharding import (broadcast_frames, exchange_halo_planes, gather_meshes, merge_slab_meshes, reshard_layers,
+from bodyslam_b200.sharding import (broadcast_frames, exchange_halo_color, exchange_halo_planes, gather_meshes, merge_slab_meshes, reshard_layers,
                                     reshard_plan, slab_bounds)
 from util import canon_mesh
 
@@ -113,6 +113,12 @@ def _worker(rank, world, port, ret):
             assert np.array_equal(lo.numpy(), tw[:, :, z0 - 1])
         if hi is not None:
             assert np.array_equal(hi.numpy(), tw[:, :, z1])
+        # colour of the bottom plane goes to rank - 1 only (its top-plane z-edges interpolate towards it)
+        rgb = np.random.default_rng(9).uniform(0, 255, size=(40, 40, 40, 3)).astype(np.float32)
+        hi_col = exchange_halo_color(torch.from_numpy(rgb[:, :, z0].copy()), rank, world)
+        assert (hi_col is None) == (rank == world - 1)
+        if hi_col is not None:
+            assert np.array_equal(hi_col.numpy(), rgb[:, :, z1])
         # frame broadcast from rank 0
         depth = torch.full((2, 4, 5), float(rank))
         color = torch.full((2, 4, 5, 3), rank, dtype=torch.uint8)
