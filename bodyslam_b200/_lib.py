@@ -69,6 +69,13 @@ _SIGNATURES = {
     "bslam_vbg_raycast_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "bslam_vbg_raycast": (C.c_int, [_p, _p, C.c_int, C.c_int, _p, _p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                     _p, _p, _p, _p, _p, _p]),
+    "bslam_odom_frame_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "bslam_odom_prepare": (C.c_int, [_p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _p, C.c_float, C.c_float, C.c_float, _p, _p]),
+    "bslam_odom_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "bslam_odom_track": (C.c_int, [_p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, _p, C.c_int, _p, _p, _p, C.c_float, C.c_float,
+                                   C.c_float, _p, _p, _p, _p, _p, _p, _p]),
+    "bslam_odom_linearize": (C.c_int, [_p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _p, C.c_int, C.c_float, C.c_float,
+                                       C.c_float, _p, _p, _p, _p]),
     "bslam_tsdf_set_extract_flavour": (C.c_int, [_p, C.c_float, C.c_double]),
     "bslam_points_set_incremental": (C.c_int, [_p, C.c_int, C.c_int]),
     "bslam_points_last_stats": (C.c_int, [_p, _p]),

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbodyslam_b200.so")
-SOURCES = ["bslam_tsdf.cu", "bslam_image.cu", "bslam_colorize_f32.cu", "bslam_extract.cu", "bslam_vbg.cu", "bslam_raycast.cu"]
+SOURCES = ["bslam_tsdf.cu", "bslam_image.cu", "bslam_colorize_f32.cu", "bslam_extract.cu", "bslam_vbg.cu", "bslam_raycast.cu", "bslam_odometry.cu"]
 
 
 def nvcc_path() -> str:

@@ -19,6 +19,7 @@ import numpy as np
 
 from . import _lib, ops
 from .geometry import PointCloud, TriangleMesh, intrinsic_params, to_numpy
+from .odometry import Method
 
 
 class DenseTSDFVolume:
@@ -848,6 +849,27 @@ class MAP:
                                                 _lib.ptr(out["vertex"]), _lib.ptr(out["normal"]), _lib.ptr(out.get("color")), _lib.ptr(self._range_ws),
                                                 _lib.stream_ptr(vol.device)))
         return out
+
+    def track_frame_to_model(self, input_rgbd, model_frame, depth_scale=None, depth_max: float = 3.0, depth_diff: float = 0.07, method=Method.PointToPlane,
+                             criteria=(6, 3, 1)):
+        """Open3D `Model.track_frame_to_model`: `odometry.rgbd_odometry_multi_scale` from the input frame (`.o3d_t_depth`,
+        `.o3d_t_color`, as `integrate` reads them) to `model_frame`, the dict `synthesize_model_frame` returns, from the
+        identity, with OdometryLossParams(depth_diff) and criteria = max iterations per level, coarsest first.
+        depth_scale None = the map's.  -> OdometryResult; compose
+        `T_frame_to_model = T_frame_to_model @ result.transformation`."""
+        from . import odometry as od
+        from .geometry import RGBDImage
+
+        method = Method(method)
+        needs_color = method != Method.PointToPlane
+        src = RGBDImage(input_rgbd.o3d_t_color if needs_color else None, input_rgbd.o3d_t_depth)
+        depth = model_frame["depth"]
+        color = model_frame.get("color") if needs_color else None
+        tgt = RGBDImage(None if color is None else color.reshape(color.shape[-3:]), depth.reshape(depth.shape[-2:]))
+        K = np.array([[self._K[0], 0.0, self._K[2]], [0.0, self._K[1], self._K[3]], [0.0, 0.0, 1.0]])
+        return od.rgbd_odometry_multi_scale(src, tgt, K, depth_scale=self.depth_scale if depth_scale is None else float(depth_scale),
+                                            depth_max=depth_max, criteria_list=[od.OdometryConvergenceCriteria(int(c)) for c in criteria],
+                                            method=method, params=od.OdometryLossParams(depth_diff))
 
     def allocated_blocks(self, last_frame: bool = False):
         """bool CUDA tensor [nbx, nby, nbz] of the 16^3 blocks of the box: activated by any frame integrated so far (the

@@ -371,6 +371,49 @@ BSLAM_API int bslam_vbg_raycast(bslam_volume *vol, const void *d_vbg_workspace, 
                                 float *d_depth, float *d_vertex, float *d_normal, float *d_color, void *d_range_workspace,
                                 bslam_stream_t stream);
 
+/* ------------------------------------------------------------------ multi-scale RGB-D odometry (row f4)
+ * Open3D's tensor `t.pipelines.odometry.rgbd_odometry_multi_scale` (the reference's `_compute_vo_o3d`,
+ * N/3DM/visual_odometry.py:97-120) and `t.pipelines.slam.Model.track_frame_to_model` (the same with the ray-cast model
+ * frame as the target): point-to-plane (method 0), intensity (1) and hybrid (2) Gauss-Newton over an image pyramid.
+ * The semantics are written down in the CPU reference tests/odometry_ref.c; they are restated from knowledge of Open3D,
+ * so parity with Open3D itself is UNPINNED (DESIGN.md section 7 lists the recalled details the reference fixes).
+ * Sums are float64 and reduced in a fixed order: the result is bit-reproducible (Open3D uses float32 atomics).
+ *
+ * Levels: level l is (H >> l) x (W >> l) with intrinsics K / 2^l; every level must be at least 1 x 1 (levels <= 16).
+ * h_K: fx, fy, cx, cy (f64) of level 0.
+ *
+ * bslam_odom_prepare: F frames -> d_frames (F * bslam_odom_frame_bytes(H, W, levels), caller-owned).  d_depth [F][H][W]
+ * uint16 (depth_dtype 0) or float32 (1), depth = raw / depth_scale, NaN (invalid) when <= 0 or >= depth_max;
+ * d_color NULL or [F][H][W][3] uint8 (color_dtype 0, intensity = (0.299 R + 0.587 G + 0.114 B) / 255) or float32 in
+ * [0, 1] (1, no division).  Without colour the intensity is NaN: such frames serve PointToPlane only (the intensity
+ * methods find no inlier on them and end singular).  Depth pyramid: PyrDownDepth(2 * depth_outlier_trunc); intensity:
+ * 5x5 Gaussian, replicated borders.  Per frame and level (coarser after finer) 12 planes of (H >> l) * (W >> l) f32:
+ * depth, intensity, vertex x, y, z, normal x, y, z, Sobel x / y of depth, Sobel x / y of intensity (unscaled 3x3).
+ *
+ * bslam_odom_track: P pairs {source, target} (h_pairs [P][2], frame indices of d_frames), each from h_init [P][16]
+ * (row-major f64, source -> target).  Levels run coarsest first; criteria entry c (h_max_iter / h_rel_fitness /
+ * h_rel_rmse [levels]) belongs to level levels - 1 - c.  Outputs: d_T [P][16] f64, d_rmse_fitness [P][2] f64 of the last
+ * evaluation, d_iters [P][levels] i32 evaluations per criteria entry, d_status [P] i32 (0 = ok, 1 = a singular 6x6
+ * system ended the pair; T is the pose before it).  d_workspace: bslam_odom_workspace_bytes(P, H, W, levels).
+ * Enqueues 2 * sum(h_max_iter) launches (+ 1 per 128 pairs); no host synchronisation, no copies.  F <= 65535 frames per
+ * bslam_odom_prepare call and P <= 65535 pairs per bslam_odom_track / bslam_odom_linearize call (E_ARG beyond).  P == 0 or F == 0
+ * (then P must be 0) launches nothing and accepts NULL outputs.
+ *
+ * bslam_odom_linearize: the 29 float64 sums of every pair at `level` under h_T [P][16]: d_sums [P][29] = upper
+ * triangle of J^T J (row-major, 21), J^T huber'(r) (6), sum of huber(r), inlier count. */
+BSLAM_API size_t bslam_odom_frame_bytes(int H, int W, int levels);
+BSLAM_API int bslam_odom_prepare(const void *d_depth, int depth_dtype, const void *d_color, int color_dtype, int F, int H, int W, int levels,
+                                 const double *h_K, float depth_scale, float depth_max, float depth_outlier_trunc, float *d_frames,
+                                 bslam_stream_t stream);
+BSLAM_API size_t bslam_odom_workspace_bytes(int P, int H, int W, int levels);
+BSLAM_API int bslam_odom_track(const float *d_frames, int F, const int *h_pairs, int P, int H, int W, int levels, const double *h_K, int method,
+                               const int *h_max_iter, const double *h_rel_fitness, const double *h_rel_rmse, float depth_outlier_trunc,
+                               float depth_huber_delta, float intensity_huber_delta, const double *h_init, double *d_T, double *d_rmse_fitness,
+                               int *d_iters, int *d_status, void *d_workspace, bslam_stream_t stream);
+BSLAM_API int bslam_odom_linearize(const float *d_frames, int F, const int *h_pairs, int P, int H, int W, int levels, int level, const double *h_K,
+                                   int method, float depth_outlier_trunc, float depth_huber_delta, float intensity_huber_delta, const double *h_T,
+                                   double *d_sums, void *d_workspace, bslam_stream_t stream);
+
 /* Surface-extraction flavour of bslam_mc_* / bslam_points_*: a voxel is valid when weight >= weight_threshold
  * (0 = weight > 0, Open3D's legacy `weight != 0` for every weight an integrator writes: they differ only for negative
  * or NaN weights, which count as invalid here; the tensor pipeline's extract_triangle_mesh / extract_point_cloud default
