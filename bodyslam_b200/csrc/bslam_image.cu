@@ -8,7 +8,6 @@
 //   a4  N/3DM/slam_utils.py:212-220,231-233
 //   K2  N/3DM/scaling_system.py:72-77, N/3DM/mapping_module.py:37,41
 #include <math.h>
-#include <stdlib.h>
 
 #include "bslam_common.cuh"
 
@@ -41,14 +40,13 @@ constexpr int kHistThreads = 256;
 constexpr int kPxPerThread = 16;
 constexpr int kPxPerBlock = kHistThreads * kPxPerThread;
 constexpr int kWindow = 4096;
-constexpr int kHistMergeDefault = 2;
 
-// MERGE: how equal values are combined before they reach the shared-memory atomics (<= 2 lanes per cycle and SM, so
-// smooth images must not spend one atomic per pixel):
-//   0 = run-length merge over the thread's 16 pixels (17 compare / flush sites; issue-bound at ~50 instructions per pixel);
-//   1 = one atomic per 4-pixel group when its pixels are equal, else one per pixel (16-byte zero / flush of the window);
-//   2 = 1 + the equal groups of a warp are combined with match.any (one atomic per distinct value and warp).
-template <bool FROM_FLOAT, int MERGE>
+// Equal values are combined before they reach the shared-memory atomics (<= 2 lanes per cycle and SM, so smooth images must
+// not spend one atomic per pixel): a 4-pixel group whose pixels are equal adds once, and the equal groups of a warp that hold
+// the same value are combined with match.any into one atomic per distinct value and warp.  The window is zeroed and
+// flushed 16 bytes at a time.  The run-length merge and the group merge without match.any measured slower:
+// profiles/r02_k1_hist_merge.md.
+template <bool FROM_FLOAT>
 __global__ void __launch_bounds__(kHistThreads) scale_hist_kernel(const float *__restrict__ depth_m, const uint16_t *__restrict__ u16_in,
                                                                    uint16_t *__restrict__ u16_out, int64_t n_per_image, float scale_mul,
                                                                    int has_invalid, unsigned int invalid_val, void *ws) {
@@ -57,11 +55,7 @@ __global__ void __launch_bounds__(kHistThreads) scale_hist_kernel(const float *_
     const int b = blockIdx.y;
     const int64_t start = (int64_t)blockIdx.x * kPxPerBlock;
     unsigned int *hist = ws_hist(ws, b);
-    if (MERGE == 0) {
-        for (int i = threadIdx.x; i < kWindow; i += kHistThreads) s_hist[i] = 0;
-    } else {
-        for (int i = threadIdx.x; i < kWindow / 4; i += kHistThreads) reinterpret_cast<uint4 *>(s_hist)[i] = make_uint4(0, 0, 0, 0);
-    }
+    for (int i = threadIdx.x; i < kWindow / 4; i += kHistThreads) reinterpret_cast<uint4 *>(s_hist)[i] = make_uint4(0, 0, 0, 0);
     if (threadIdx.x == 0) s_min = 0xffffffffu;
     __syncthreads();
 
@@ -71,7 +65,7 @@ __global__ void __launch_bounds__(kHistThreads) scale_hist_kernel(const float *_
     // a value no pixel can hold when there is no invalid marker: one compare + select per pixel either way
     const unsigned int inv = has_invalid ? invalid_val : 0xfffffffeu;
     // thread t handles 4 groups of 4 consecutive pixels, groups strided by 1024 -> 16-byte accesses
-    if (MERGE != 0 && start + kPxPerBlock <= n_per_image && ((img_off + start) & 3) == 0) {
+    if (start + kPxPerBlock <= n_per_image && ((img_off + start) & 3) == 0) {
         // the whole block lies inside the image and its rows of 4 are 16-byte aligned: no per-group tests
         const int64_t q = img_off + start + threadIdx.x * 4;
 #pragma unroll
@@ -140,30 +134,6 @@ __global__ void __launch_bounds__(kHistThreads) scale_hist_kernel(const float *_
     __syncthreads();
     const unsigned int base = s_min;
     if (base == 0xffffffffu) return; // no valid pixel in this block
-    if (MERGE == 0) {
-        // run-length merge inside the thread, then shared (window) or global atomics
-        unsigned int run_v = 0xffffffffu, run_n = 0;
-#pragma unroll
-        for (int i = 0; i <= kPxPerThread; ++i) {
-            const unsigned int x = (i < kPxPerThread) ? val[i] : 0xffffffffu;
-            if (x == run_v && x != 0xffffffffu) {
-                ++run_n;
-            } else {
-                if (run_n) {
-                    const unsigned int rel = run_v - base;
-                    if (rel < kWindow) atomicAdd(&s_hist[rel], run_n);
-                    else atomicAdd(&hist[run_v], run_n);
-                }
-                run_v = x; run_n = (x != 0xffffffffu) ? 1u : 0u;
-            }
-        }
-        __syncthreads();
-        for (int i = threadIdx.x; i < kWindow; i += kHistThreads) {
-            const unsigned int c = s_hist[i];
-            if (c) atomicAdd(&hist[base + i], c);
-        }
-        return;
-    }
     // the marker 0xffffffff never lands in the window (base <= 65535), so only the global path tests for it
     auto add = [&](unsigned int x, unsigned int n) {
         const unsigned int rel = x - base;
@@ -178,15 +148,10 @@ __global__ void __launch_bounds__(kHistThreads) scale_hist_kernel(const float *_
     for (int g = 0; g < kPxPerThread / 4; ++g) {
         const unsigned int a = val[4 * g], c1 = val[4 * g + 1], c2 = val[4 * g + 2], c3 = val[4 * g + 3];
         const bool uni = (a == c1) & (c1 == c2) & (c2 == c3);
-        if (MERGE == 2) {
-            // lanes whose group is equal AND holds the same value elect their lowest lane; a mixed group matches nobody
-            const unsigned int peers = __match_any_sync(0xffffffffu, uni ? a : (0xffff0000u | (threadIdx.x & 31)));
-            if (uni) {
-                if ((threadIdx.x & 31) == __ffs(peers) - 1) add(a, 4u * __popc(peers));
-                continue;
-            }
-        } else if (uni) {
-            add(a, 4u);
+        // lanes whose group is equal AND holds the same value elect their lowest lane; a mixed group matches nobody
+        const unsigned int peers = __match_any_sync(0xffffffffu, uni ? a : (0xffff0000u | (threadIdx.x & 31)));
+        if (uni) {
+            if ((threadIdx.x & 31) == __ffs(peers) - 1) add(a, 4u * __popc(peers));
             continue;
         }
         add(a, one); add(c1, one); add(c2, one); add(c3, one);
@@ -719,20 +684,8 @@ static int run_hist(const float *d_depth_m, const uint16_t *d_u16_in, int B, int
                     int has_invalid, uint16_t invalid_val, void *ws, cudaStream_t st) {
     BSLAM_CUDA(cudaMemsetAsync(ws, 0, bslam_colorize_workspace_bytes(B), st));
     const dim3 grid((unsigned)((n + kPxPerBlock - 1) / kPxPerBlock), (unsigned)B);
-    static const int merge = [] {   // BSLAM_K1_MERGE = 0 | 1 | 2 selects the merge scheme (measurement switch; same histogram either way)
-        const char *e = getenv("BSLAM_K1_MERGE");
-        const int m = e ? atoi(e) : kHistMergeDefault;
-        return (m >= 0 && m <= 2) ? m : kHistMergeDefault;
-    }();
-#define BSLAM_HIST(M_)                                                                                                                       \
-    do {                                                                                                                                     \
-        if (d_depth_m) scale_hist_kernel<true, M_><<<grid, kHistThreads, 0, st>>>(d_depth_m, nullptr, d_u16_out, n, scale_mul, has_invalid, invalid_val, ws); \
-        else scale_hist_kernel<false, M_><<<grid, kHistThreads, 0, st>>>(nullptr, d_u16_in, nullptr, n, scale_mul, has_invalid, invalid_val, ws);             \
-    } while (0)
-    if (merge == 0) BSLAM_HIST(0);
-    else if (merge == 1) BSLAM_HIST(1);
-    else BSLAM_HIST(2);
-#undef BSLAM_HIST
+    if (d_depth_m) scale_hist_kernel<true><<<grid, kHistThreads, 0, st>>>(d_depth_m, nullptr, d_u16_out, n, scale_mul, has_invalid, invalid_val, ws);
+    else scale_hist_kernel<false><<<grid, kHistThreads, 0, st>>>(nullptr, d_u16_in, nullptr, n, scale_mul, has_invalid, invalid_val, ws);
     BSLAM_LAUNCH_CHECK();
     return BSLAM_OK;
 }

@@ -325,11 +325,10 @@ class ShardedTSDF:
         import torch
         import torch.distributed as dist
 
-        from .geometry import intrinsic_params, to_numpy
+        from .geometry import to_numpy
 
         vol = self.tsdf
         dev = vol.device
-        W, H = intrinsic_params(intrinsic)[:2]
         E = np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4)
         F = E.shape[0]
         on_dev = bool(getattr(depth_u16, "is_cuda", False))
@@ -345,12 +344,8 @@ class ShardedTSDF:
         if vol.color:
             raise RuntimeError("integrate_stream: colour volumes are not streamed yet (use integrate_batch)")
         is_src = self.rank == src
-        from_host = is_src and not depth_u16.is_cuda
         with torch.cuda.device(dev):
-            main = torch.cuda.current_stream(dev)
-            if getattr(self, "_copy_stream", None) is None:
-                self._copy_stream = torch.cuda.Stream(dev)
-            cs = self._copy_stream
+            cs = vol.copy_stream()
             with torch.cuda.stream(cs):                           # poses (128 B per frame), off the compute stream
                 hdr = torch.cat([torch.as_tensor(E).reshape(-1), torch.tensor([1.0 if on_dev else 0.0], dtype=torch.float64)])
                 hdr = hdr.to(dev, non_blocking=True)
@@ -358,58 +353,26 @@ class ShardedTSDF:
                 hdr = hdr.cpu().numpy()                           # the C ABI takes the poses from host memory
             E, src_on_dev = hdr[:-1].reshape(-1, 4, 4), bool(hdr[-1] != 0.0)
             chunks = vol.stream_chunks(F, chunk, ramp=self.stream_ramp(self.world_size, src_on_dev))
-            n = max(f1 - f0 for f0, f1 in chunks)
-            stage = vol._staging(n, H, W, False, count=3)
-            free = vol._stage_free                                # kept across calls (see DenseTSDFVolume._staging)
-
-            dev_src = is_src and not from_host                    # frames already in this rank's HBM: broadcast them in place
+            dev_src = is_src and depth_u16.is_cuda                # frames already in this rank's HBM: broadcast them in place
             if dev_src:
-                cs.wait_stream(main)                              # whoever produced them did so on the current stream
-            bufs = {}
+                cs.wait_stream(torch.cuda.current_stream(dev))    # whoever produced them did so on the current stream
 
-            def issue(k):
+            def arrive(k, stage, free):
                 f0, f1 = chunks[k]
-                m = f1 - f0
                 with torch.cuda.stream(cs):
                     if dev_src:
                         u16 = depth_u16[f0:f1]
                     else:
-                        u16 = stage[k % 3][0][:m]
-                        if free[k % 3] is not None:
-                            cs.wait_event(free[k % 3])
+                        u16 = stage[0][:f1 - f0]
+                        cs.wait_event(free)
                         if is_src:
                             u16.copy_(depth_u16[f0:f1], non_blocking=True)
-                    bufs[k] = u16
                     # the collective is enqueued behind the copy stream's work (NCCL waits for the
                     # stream that is current at the call); NCCL has no 16-bit integer type: ship bytes
-                    return dist.broadcast(u16.view(torch.uint8), src, group=self.group, async_op=True)
+                    work = dist.broadcast(u16.view(torch.uint8), src, group=self.group, async_op=True)
+                return u16, None, work.wait
 
-            pipelined = vol.pipeline_enabled()
-            if pipelined:
-                vol.prep_stream().wait_stream(main)
-
-            def prep(k):     # conversion + statistics + culling of chunk k on the side stream, once its frames have arrived
-                f0, f1 = chunks[k]
-                vol.prepare_u16(bufs.pop(k), intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc, wait=works.pop(k).wait)
-
-            works = {0: issue(0)}
-            if len(chunks) > 1:
-                works[1] = issue(1)
-            if pipelined:
-                prep(0)
-            for k, (f0, f1) in enumerate(chunks):
-                if k + 2 < len(chunks):
-                    works[k + 2] = issue(k + 2)
-                cnt = None if update_counts is None else update_counts[f0:f1]
-                if pipelined:
-                    if k + 1 < len(chunks):
-                        prep(k + 1)                                # overlaps the integration of chunk k
-                    vol.integrate_prepared(None, cnt)
-                else:
-                    works.pop(k).wait()                            # current stream waits for chunk k
-                    vol.integrate_u16_batch(bufs.pop(k), None, intrinsic, E[f0:f1], depth_scale, depth_trunc, scratch=stage[k % 3][1], update_counts=cnt)
-                free[k % 3] = torch.cuda.Event()
-                free[k % 3].record(main)
+            vol.integrate_streamed(chunks, intrinsic, E, arrive, depth_scale, depth_trunc, update_counts)
 
     # ------------------------------------------------------------------ sharded ingest
     @staticmethod
@@ -442,12 +405,11 @@ class ShardedTSDF:
         import torch
         import torch.distributed as dist
 
-        from .geometry import intrinsic_params, to_numpy
+        from .geometry import to_numpy
 
         vol = self.tsdf
         dev = vol.device
         N, rank = self.world_size, self.rank
-        W, H = intrinsic_params(intrinsic)[:2]
         E = np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4)
         F = E.shape[0]
         if N == 1:
@@ -457,26 +419,19 @@ class ShardedTSDF:
         chunks, pieces = self.ingest_pieces(F, N, chunk)
         if depth_u16_share.shape[0] != sum(pc[rank][1] - pc[rank][0] for pc in pieces):
             raise RuntimeError("integrate_stream_sharded: this rank's share does not match ingest_share(F, rank, world_size, chunk)")
-        n = max(f1 - f0 for f0, f1 in chunks)
         with torch.cuda.device(dev):
-            main = torch.cuda.current_stream(dev)
-            if getattr(self, "_copy_stream", None) is None:
-                self._copy_stream = torch.cuda.Stream(dev)
-            cs = self._copy_stream
-            stage = vol._staging(n, H, W, False, count=3)
-            free = vol._stage_free
+            cs = vol.copy_stream()
             if depth_u16_share.is_cuda:
-                cs.wait_stream(main)
+                cs.wait_stream(torch.cuda.current_stream(dev))
             offs = np.concatenate([[0], np.cumsum([pc[rank][1] - pc[rank][0] for pc in pieces])])
 
-            def issue(k):
+            def arrive(k, stage, free):
                 f0, f1 = chunks[k]
-                u16 = stage[k % 3][0][:f1 - f0]
+                u16 = stage[0][:f1 - f0]
                 a, b = pieces[k][rank]
                 works = []
                 with torch.cuda.stream(cs):
-                    if free[k % 3] is not None:
-                        cs.wait_event(free[k % 3])
+                    cs.wait_event(free)
                     if b > a:
                         u16[a - f0:b - f0].copy_(depth_u16_share[offs[k]:offs[k + 1]], non_blocking=True)
                     sizes = {q1 - q0 for q0, q1 in pieces[k]}
@@ -487,38 +442,9 @@ class ShardedTSDF:
                         for q, (q0, q1) in enumerate(pieces[k]):
                             if q1 > q0:
                                 works.append(dist.broadcast(u8[q0 - f0:q1 - f0], q, group=self.group, async_op=True))
-                return works
+                return u16, None, lambda: [w.wait() for w in works]
 
-            pipelined = vol.pipeline_enabled()
-            if pipelined:
-                vol.prep_stream().wait_stream(main)
-
-            def prep(k):
-                f0, f1 = chunks[k]
-                ws = pending.pop(k)
-                vol.prepare_u16(stage[k % 3][0][:f1 - f0], intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc,
-                                wait=lambda: [w.wait() for w in ws])
-
-            pending = {0: issue(0)}
-            if len(chunks) > 1:
-                pending[1] = issue(1)
-            if pipelined:
-                prep(0)
-            for k, (f0, f1) in enumerate(chunks):
-                if k + 2 < len(chunks):
-                    pending[k + 2] = issue(k + 2)
-                cnt = None if update_counts is None else update_counts[f0:f1]
-                if pipelined:
-                    if k + 1 < len(chunks):
-                        prep(k + 1)                                  # overlaps the integration of chunk k
-                    vol.integrate_prepared(None, cnt)
-                else:
-                    for w in pending.pop(k):
-                        w.wait()                                     # current stream waits for chunk k
-                    vol.integrate_u16_batch(stage[k % 3][0][:f1 - f0], None, intrinsic, E[f0:f1], depth_scale, depth_trunc,
-                                            scratch=stage[k % 3][1], update_counts=cnt)
-                free[k % 3] = torch.cuda.Event()
-                free[k % 3].record(main)
+            vol.integrate_streamed(chunks, intrinsic, E, arrive, depth_scale, depth_trunc, update_counts)
 
     def build_3D_map(self, rgbd, intrinsic, extrinsic):
         self.tsdf.integrate(rgbd, intrinsic, extrinsic)

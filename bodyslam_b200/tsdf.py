@@ -13,7 +13,6 @@ from __future__ import annotations
 
 import copy as _copy
 import ctypes as C
-import os
 
 import numpy as np
 
@@ -212,18 +211,19 @@ class DenseTSDFVolume:
         return scratch
 
     # ------------------------------------------------------------------ two-stream launch pipeline
-    @staticmethod
-    def pipeline_enabled() -> bool:
-        """BODYSLAM_PIPELINE=0 makes the streamed entry points run preparation and integration back to back on one
-        stream (measurement switch; the default overlaps the preparation of chunk k+1 with the integration of chunk k)"""
-        return os.environ.get("BODYSLAM_PIPELINE", "1") != "0"
-
     def prep_stream(self):
         """side stream for the part of a launch that does not touch the volume (conversion, statistics, culling)"""
         torch = _lib.require_cuda()
         if getattr(self, "_prep_stream", None) is None:
             self._prep_stream = torch.cuda.Stream(self.device)
         return self._prep_stream
+
+    def copy_stream(self):
+        """side stream on which the streamed entry points bring frames to the device (host copies, NCCL transfers)"""
+        torch = _lib.require_cuda()
+        if getattr(self, "_copy_stream", None) is None:
+            self._copy_stream = torch.cuda.Stream(self.device)
+        return self._copy_stream
 
     def prepare_u16(self, depth_u16, intrinsic, extrinsics, scratch, depth_scale: float = 1000.0, depth_trunc: float = 3.0, wait=None):
         """enqueue the preparation of one launch (<= 256 frames; see bslam_tsdf_prepare_u16) on the side stream.
@@ -263,33 +263,54 @@ class DenseTSDFVolume:
                                                              _lib.stream_ptr(self.device)))
         self.frames_integrated += F
 
+    def integrate_streamed(self, chunks, intrinsic, extrinsics, arrive, depth_scale: float = 1000.0, depth_trunc: float = 3.0,
+                           update_counts=None, color_staging: bool = False):
+        """The two-stream launch pipeline that every streamed entry point runs, chunk k of `chunks` [(f0, f1)] after
+        chunk k-1: the arrival of chunk k+2 is enqueued, then the preparation of chunk k+1 on the side stream, then the
+        integration of chunk k on the current stream.  The caller says how frames arrive:
+            arrive(k, stage, free) -> (depth_u16, color, wait)
+        enqueues the arrival of chunk k.  `stage` = (uint16 [n,H,W], f32 [n,H,W], uint8 [n,H,W,3] | None) are the
+        staging buffers chunk k may use (the f32 one always receives its converted frames), `free` is the event after
+        which the current stream no longer reads them.  It returns the chunk's uint16 frames on the device, its colour
+        (or None) and the callable the side stream runs before the preparation (or None)."""
+        torch = _lib.require_cuda()
+        if not chunks:
+            return
+        W, H = intrinsic_params(intrinsic)[:2]
+        E = np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4)
+        with torch.cuda.device(self.device):
+            main = torch.cuda.current_stream(self.device)
+            stage = self._staging(max(f1 - f0 for f0, f1 in chunks), H, W, color_staging)
+            free = self._stage_free
+            self.prep_stream().wait_stream(main)         # the frames (and earlier launches) are ordered by the current stream
+            arrived = {}
+
+            def prep(k):
+                f0, f1 = chunks[k]
+                self.prepare_u16(arrived[k][0], intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc, wait=arrived[k][2])
+
+            for k in range(min(2, len(chunks))):
+                arrived[k] = arrive(k, stage[k % 3], free[k % 3])
+            prep(0)
+            for k, (f0, f1) in enumerate(chunks):
+                if k + 2 < len(chunks):
+                    arrived[k + 2] = arrive(k + 2, stage[(k + 2) % 3], free[(k + 2) % 3])
+                if k + 1 < len(chunks):
+                    prep(k + 1)
+                self.integrate_prepared(arrived.pop(k)[1], None if update_counts is None else update_counts[f0:f1])
+                free[k % 3] = torch.cuda.Event()
+                free[k % 3].record(main)
+
     def integrate_u16_chunks(self, depth_u16, color, intrinsic, extrinsics, chunks, depth_scale: float = 1000.0, depth_trunc: float = 3.0,
                              update_counts=None):
         """device-resident uint16 frames, launch after launch through the two-stream pipeline: chunk k+1 is converted and
         culled on the side stream while chunk k integrates (`chunks`: [(f0, f1)], each <= 256 frames)."""
-        torch = _lib.require_cuda()
-        E = np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4)
-        if not chunks:
-            return
-        if not self.pipeline_enabled():
-            for f0, f1 in chunks:
-                self.integrate_u16_batch(depth_u16[f0:f1], None if color is None else color[f0:f1], intrinsic, E[f0:f1], depth_scale, depth_trunc,
-                                         update_counts=None if update_counts is None else update_counts[f0:f1])
-            return
-        H, W = depth_u16.shape[1], depth_u16.shape[2]
-        stage = self._staging(max(f1 - f0 for f0, f1 in chunks), H, W, False, count=3)
-        main = torch.cuda.current_stream(self.device)
-        self.prep_stream().wait_stream(main)             # the frames (and earlier launches) are ordered by the current stream
 
-        def prep(k):
+        def arrive(k, stage, free):      # already on the device and ordered by the current stream
             f0, f1 = chunks[k]
-            self.prepare_u16(depth_u16[f0:f1], intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc)
+            return depth_u16[f0:f1], None if color is None else color[f0:f1], None
 
-        prep(0)
-        for k, (f0, f1) in enumerate(chunks):
-            if k + 1 < len(chunks):
-                prep(k + 1)
-            self.integrate_prepared(None if color is None else color[f0:f1], None if update_counts is None else update_counts[f0:f1])
+        self.integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts)
 
     @staticmethod
     def stream_chunks(F: int, chunk: int = 256, ramp=(32, 64, 128), multiple_of: int = 1):
@@ -352,56 +373,25 @@ class DenseTSDFVolume:
             depth_u16 = torch.from_numpy(np.ascontiguousarray(to_numpy(depth_u16)))
         if color is not None and not hasattr(color, "is_cuda"):
             color = torch.from_numpy(np.ascontiguousarray(to_numpy(color)))
-        F, H, W = depth_u16.shape
-        E = np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4)
         use_color = self.color and color is not None
         if self.color and color is None:
             raise RuntimeError("[DenseTSDFVolume::IntegrateHost] Unsupported image format.")
-        dev = self.device
-        with torch.cuda.device(dev):
-            main = torch.cuda.current_stream(dev)
-            if getattr(self, "_copy_stream", None) is None:
-                self._copy_stream = torch.cuda.Stream(dev)
-            cs = self._copy_stream
-            chunks = self.stream_chunks(F, chunk)
-            stage = self._staging(max(f1 - f0 for f0, f1 in chunks), H, W, use_color, count=3)
-            free = self._stage_free  # event: the compute stream is done with staging buffer i
-            ps = self.prep_stream()
-            ps.wait_stream(main)
-            copied = {}
+        chunks = self.stream_chunks(depth_u16.shape[0], chunk)
+        cs = self.copy_stream()
 
-            def copy(k):                 # H2D of chunk k on the copy stream
-                f0, f1 = chunks[k]
-                m = f1 - f0
-                u16, _, col = stage[k % 3]
-                with torch.cuda.stream(cs):
-                    if free[k % 3] is not None:
-                        cs.wait_event(free[k % 3])
-                    u16[:m].copy_(depth_u16[f0:f1], non_blocking=True)
-                    if use_color:
-                        col[:m].copy_(color[f0:f1], non_blocking=True)
-                    copied[k] = torch.cuda.Event()
-                    copied[k].record(cs)
+        def arrive(k, stage, free):      # H2D of chunk k on the copy stream, once the current stream is done with its buffers
+            f0, f1 = chunks[k]
+            u16, _, col = stage
+            with torch.cuda.stream(cs):
+                cs.wait_event(free)
+                u16[:f1 - f0].copy_(depth_u16[f0:f1], non_blocking=True)
+                if use_color:
+                    col[:f1 - f0].copy_(color[f0:f1], non_blocking=True)
+                copied = torch.cuda.Event()
+                copied.record(cs)
+            return u16[:f1 - f0], col[:f1 - f0] if use_color else None, copied.wait
 
-            def prep(k):                 # conversion + statistics + culling of chunk k on the side stream
-                f0, f1 = chunks[k]
-                ev = copied.pop(k)
-                self.prepare_u16(stage[k % 3][0][:f1 - f0], intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc,
-                                 wait=lambda: ps.wait_event(ev))
-
-            copy(0)
-            if len(chunks) > 1:
-                copy(1)
-            prep(0)
-            for k, (f0, f1) in enumerate(chunks):
-                if k + 2 < len(chunks):
-                    copy(k + 2)
-                if k + 1 < len(chunks):
-                    prep(k + 1)
-                col = stage[k % 3][2]
-                self.integrate_prepared(col[:f1 - f0] if use_color else None, None if update_counts is None else update_counts[f0:f1])
-                free[k % 3] = torch.cuda.Event()
-                free[k % 3].record(main)
+        self.integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts, use_color)
 
     def count_updates(self, depth, intrinsic, extrinsics, zmarch: int = _lib.ZMARCH_BRICK):
         """U_f of SURVEY.md 8(d): voxels each frame WOULD update (volume untouched) -> i64 [F]."""
