@@ -408,9 +408,10 @@ class DenseTSDFVolume:
 
     def dry_stats(self, reset: bool = True):
         """culling statistics of the dry runs since the last reset (see bslam_tsdf_dry_stats) -> dict"""
-        out = (C.c_ulonglong * 4)()
+        out = (C.c_ulonglong * 5)()
         _lib.check(self._L.bslam_tsdf_dry_stats(self._h, out, int(bool(reset)), _lib.stream_ptr(self.device)))
-        return {"warp_frame_pairs": int(out[0]), "pairs_in_image": int(out[1]), "pairs_updating": int(out[2]), "voxels_tested": int(out[3])}
+        return {"warp_frame_pairs": int(out[0]), "pairs_in_image": int(out[1]), "pairs_updating": int(out[2]), "voxels_tested": int(out[3]),
+                "free_pairs": int(out[4])}
 
     def chain_histogram(self):
         """active bricks of the last integrate launch by number of active frames (32 buckets of 8 frames)"""

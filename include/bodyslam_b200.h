@@ -258,9 +258,10 @@ BSLAM_API int bslam_tsdf_chain_histogram(bslam_volume *vol, unsigned int *h_hist
 BSLAM_API int bslam_tsdf_set_z_split(bslam_volume *vol, int z_layers_per_warp);
 
 /* Culling statistics accumulated by dry runs (bslam_tsdf_integrate with dry_run = 1) since the last
- * reset: h_stat4 = {(warp, frame) pairs tested, pairs with a voxel projecting into the image, pairs
- * with an updated voxel, voxels tested}.  Measurement aid for DESIGN.md / bench.py; synchronises. */
-BSLAM_API int bslam_tsdf_dry_stats(bslam_volume *vol, unsigned long long *h_stat4, int reset, bslam_stream_t stream);
+ * reset: h_stat5 = {(warp, frame) pairs tested, pairs with a voxel projecting into the image, pairs
+ * with an updated voxel, voxels tested, free pairs (the cull proved every update has t == 1)}.
+ * Measurement aid for DESIGN.md / bench.py; synchronises. */
+BSLAM_API int bslam_tsdf_dry_stats(bslam_volume *vol, unsigned long long *h_stat5, int reset, bslam_stream_t stream);
 
 /* Device self-test: n random operand triples through the kernels' shared-reciprocal division and
  * magic-number floor, compared with IEEE `/` and (int) casts; returns the number of mismatches
