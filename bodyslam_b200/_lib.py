@@ -66,6 +66,9 @@ _SIGNATURES = {
     "bslam_vbg_integrate": (C.c_int, [_p, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p, C.c_float, C.c_float, _p, _p, _p]),
     "bslam_vbg_stats": (C.c_int, [_p, _p, _p]),
     "bslam_tsdf_raycast": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, _p, _p, C.c_float, C.c_float, C.c_float, C.c_float, _p, _p, _p, _p, _p]),
+    "bslam_tsdf_raycast_halo_bytes": (C.c_size_t, [_p, C.c_int]),
+    "bslam_tsdf_raycast_segment": (C.c_int, [_p, C.c_int, _p, C.c_int, C.c_int, C.c_int, C.c_int, _p, _p, C.c_float, C.c_float, C.c_float, _p, _p]),
+    "bslam_tsdf_raycast_shade": (C.c_int, [_p, C.c_int, _p, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, C.c_float, _p, _p, _p, _p, _p, _p]),
     "bslam_vbg_raycast_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "bslam_vbg_raycast": (C.c_int, [_p, _p, C.c_int, C.c_int, _p, _p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                     _p, _p, _p, _p, _p, _p]),

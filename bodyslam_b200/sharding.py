@@ -10,6 +10,8 @@ data-path collective, and only surface extraction exchanges data:
   * a gather of the per-slab meshes to rank 0, where vertex ids are rebased and the references
     into the next slab's first plane are resolved -- the result equals the single-GPU mesh after
     canonical ordering.
+The ray cast (`ShardedTSDF.raycast`) marches every ray through the slabs in rounds: only the ray states
+(an all-reduce per round), one packed halo each way and the shaded maps (a reduce to one rank) cross NVLink.
 Frames reach the ranks either from each rank's own copy (synthetic / shared storage) or by a
 broadcast from rank 0 (`broadcast_frames`), which is the only NCCL traffic during integration.
 """
@@ -104,7 +106,8 @@ def broadcast_frames(depth, color, extrinsics, src: int = 0, group=None):
 
 
 def exchange_halo_planes(top_plane, bottom_plane, rank: int, world_size: int, group=None):
-    """neighbour exchange: returns (halo_lo, halo_hi) = (top plane of rank-1, bottom plane of rank+1)."""
+    """neighbour exchange: returns (halo_lo, halo_hi) = (top plane of rank-1, bottom plane of rank+1).  The "planes" are
+    any per-slab tensors of one shape per side, such as the packed halos of `DenseTSDFVolume.raycast_halo`."""
     import torch
     import torch.distributed as dist
 
@@ -467,6 +470,83 @@ class ShardedTSDF:
         for k in src:
             reshard_layers(src[k], dst[k], send, recv, self.group)
         return slab
+
+    def raycast(self, intrinsic, extrinsics, depth_min: float = 0.0, depth_max: float = 3.0, depth_scale: float = 1.0,
+                weight_threshold: float = 0.0, normals: bool = True, colors=None, dst: int = 0, broadcast_from=None, profile: bool = False):
+        """`DenseTSDFVolume.raycast` of the whole grid, bit for bit, without gathering it: rank `dst` gets the dict, the other
+        ranks None.  Every rank calls it; with `broadcast_from` only that rank needs the poses.
+        The grid is cut into contiguous slabs (re-sharded in interleaved layout).  In each round every rank marches the rays
+        it owns until they hit, leave the depth window or reach a sample of another slab, and an int32 all-reduce of the ray
+        states hands them on; at most world_size rounds, fewer when a round hands nothing over.  Each hit is shaded by the
+        slab holding its trilinear base plane (one halo plane below, two above), and the maps are summed on `dst` as
+        int32 bit patterns (every pixel has one writer).  profile=True synchronises between the phases and leaves their
+        wall-clock milliseconds and the round count in `self.last_raycast_profile` (measurement aid)."""
+        if self.world_size == 1:
+            out = self.tsdf.raycast(intrinsic, extrinsics, depth_min, depth_max, depth_scale, weight_threshold, normals, colors)
+            return out if self.rank == dst else None
+        import time
+
+        import torch
+        import torch.distributed as dist
+
+        from .geometry import intrinsic_params, to_numpy
+
+        dev, N, rank, g = self.tsdf.device, self.world_size, self.rank, self.group
+        t = [time.perf_counter()]
+
+        def mark():
+            if profile:
+                torch.cuda.synchronize(dev)
+                t.append(time.perf_counter())
+
+        if broadcast_from is not None:
+            mine = rank == broadcast_from
+            n = torch.tensor([np.asarray(to_numpy(extrinsics)).size // 16 if mine else 0], dtype=torch.int64, device=dev)
+            dist.broadcast(n, broadcast_from, group=g)
+            E = (torch.as_tensor(np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4), device=dev) if mine
+                 else torch.empty((int(n.item()), 4, 4), dtype=torch.float64, device=dev))
+            dist.broadcast(E, broadcast_from, group=g)
+            extrinsics = E.cpu().numpy()
+        E = np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 4, 4)
+        W, H = intrinsic_params(intrinsic)[:2]
+        F, n_pix = E.shape[0], E.shape[0] * H * W
+        colors = self.tsdf.color if colors is None else bool(colors)
+        v = self.contiguous_slab()
+        mark()
+        lo, hi = exchange_halo_planes(v.raycast_halo(True), v.raycast_halo(False), rank, N, g)
+        mark()
+        slab_z = np.asarray([b[0] for b in self.bounds] + [self.nz], dtype=np.int32)
+        state = torch.empty(4 * n_pix + 1, dtype=torch.int32, device=dev)
+        rounds = 0
+        while F and rounds < N:
+            v.raycast_segment(state, slab_z, rounds == 0, intrinsic, E, depth_min, depth_max, weight_threshold)
+            dist.all_reduce(state, group=g)
+            rounds += 1
+            if int(state[-1].item()) == 0:
+                break
+        else:
+            if F:
+                raise RuntimeError(f"ShardedTSDF.raycast: rays still marching after {N} rounds")
+        mark()
+        chans = {"depth": 1, "vertex": 3}
+        if normals:
+            chans["normal"] = 3
+        if colors:
+            chans["color"] = 3
+        buf = torch.empty(n_pix * sum(chans.values()), dtype=torch.int32, device=dev)
+        out, o = {}, 0
+        for k, c in chans.items():
+            out[k] = buf[o:o + c * n_pix].view(torch.float32).view((F, H, W) + ((3,) if c == 3 else ()))
+            o += c * n_pix
+        v.raycast_shade(state, slab_z, lo, hi, intrinsic, E, out, depth_scale)
+        if buf.numel():
+            dist.reduce(buf, dst, op=dist.ReduceOp.SUM, group=g)
+        mark()
+        if profile:
+            names = ("reshard_to_slabs", "halo_exchange", "rounds", "shade_and_composite")
+            self.last_raycast_profile = {n: 1e3 * (b - a) for n, a, b in zip(names, t[:-1], t[1:])}
+            self.last_raycast_profile["n_rounds"] = rounds
+        return out if rank == dst else None
 
     def extract_mesh(self, profile: bool = False):
         """full mesh on rank 0 (None on the other ranks).  profile=True synchronises between the phases and leaves

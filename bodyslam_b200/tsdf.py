@@ -527,6 +527,47 @@ class DenseTSDFVolume:
                                                   _lib.ptr(out.get("normal")), _lib.ptr(out.get("color")), _lib.stream_ptr(self.device)))
         return out
 
+    # ------------------------------------------------------------------ ray casting of z-slabs (ShardedTSDF.raycast)
+    def raycast_halo(self, up: bool):
+        """what this slab gives a neighbour for `raycast_shade`, packed as bslam_tsdf_raycast_halo_bytes bytes (uint8 CUDA
+        tensor): up=True -> its top plane for the slab above, up=False -> its two bottom planes for the slab below; each
+        with the colour planes of colour volumes and the brick flags of the layer holding them."""
+        torch = _lib.require_cuda()
+        zs = [self.nz - 1] if up else [0, 1]
+        parts = [self.export_plane(z).view(torch.uint8).reshape(-1) for z in zs]
+        if self.color:
+            parts += [self.export_plane_color(z).view(torch.uint8).reshape(-1) for z in zs]
+        parts.append(self.storage_layers()["flags"][-1 if up else 0])
+        return torch.cat(parts)
+
+    def raycast_segment(self, state, slab_z, first: bool, intrinsic, extrinsics, depth_min: float = 0.0, depth_max: float = 3.0,
+                        weight_threshold: float = 0.0):
+        """one round of the segment march on this slab of the grid cut at planes `slab_z` (bslam_tsdf_raycast_segment);
+        state: int32 CUDA tensor of 4 * F * H * W + 1 words, overwritten with this slab's share of the next state."""
+        torch = _lib.require_cuda()
+        W, H, fx, fy, cx, cy = intrinsic_params(intrinsic)
+        E = np.ascontiguousarray(np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 16))
+        z = np.ascontiguousarray(slab_z, dtype=np.int32)
+        K = np.array([fx, fy, cx, cy], dtype=np.float64)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.bslam_tsdf_raycast_segment(self._h, len(z) - 1, _lib.ptr(z), int(bool(first)), E.shape[0], H, W, _lib.ptr(K), _lib.ptr(E),
+                                                          float(depth_min), float(depth_max), float(weight_threshold), _lib.ptr(state),
+                                                          _lib.stream_ptr(self.device)))
+
+    def raycast_shade(self, state, slab_z, halo_lo, halo_hi, intrinsic, extrinsics, out, depth_scale: float = 1.0):
+        """this slab's share of the maps of the finished rays in `state` (bslam_tsdf_raycast_shade) into the tensors of
+        `out` (keys as `raycast`); halo_lo / halo_hi: `raycast_halo` of the slabs below (up=True) / above (up=False)."""
+        torch = _lib.require_cuda()
+        W, H, fx, fy, cx, cy = intrinsic_params(intrinsic)
+        E = np.ascontiguousarray(np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 16))
+        z = np.ascontiguousarray(slab_z, dtype=np.int32)
+        K = np.array([fx, fy, cx, cy], dtype=np.float64)
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.bslam_tsdf_raycast_shade(self._h, len(z) - 1, _lib.ptr(z), _lib.ptr(halo_lo), _lib.ptr(halo_hi), E.shape[0], H, W,
+                                                        _lib.ptr(K), _lib.ptr(E), float(depth_scale), _lib.ptr(state), _lib.ptr(out["depth"]),
+                                                        _lib.ptr(out.get("vertex")), _lib.ptr(out.get("normal")), _lib.ptr(out.get("color")),
+                                                        _lib.stream_ptr(self.device)))
+
     # ------------------------------------------------------------------ extraction
     def mc_count(self, halo_lo=None, halo_hi=None):
         """first phase of the marching cubes: (vertices, triangles) this box will emit (synchronises)"""

@@ -361,6 +361,30 @@ BSLAM_API int bslam_vbg_stats(const void *d_workspace, unsigned long long *h_sta
 BSLAM_API int bslam_tsdf_raycast(bslam_volume *vol, int F, int H, int W, const double *h_K, const double *h_extrinsics, float depth_scale,
                                  float depth_min, float depth_max, float weight_threshold, float *d_depth, float *d_vertex, float *d_normal,
                                  float *d_color, bslam_stream_t stream);
+/* The same legacy ray cast over a grid cut into contiguous z-slabs [h_slab_z[k], h_slab_z[k+1]) that live on different
+ * devices (ShardedTSDF.raycast); the result equals bslam_tsdf_raycast of the whole grid bit for bit.  h_slab_z: n_slabs + 1
+ * increasing global planes, multiples of 8, from 0 to the grid's z (1 <= n_slabs <= 64); vol: one of these slabs
+ * (not z-interleaved).  Rays are marched in rounds: a ray's state lives in d_state [F][H][W] int32x4 {t or the hit
+ * distance, t_prev, last tsdf, owner slab << 2 | status (1 marching, 2 hit, 3 miss)} followed by one int32, the count of
+ * rays handed to another slab in the round.
+ * bslam_tsdf_raycast_segment: one round on this slab.  first != 0: d_state is not read (every slab computes each ray's
+ * first owner itself).  Writes the state of the rays this slab owned and 0 for all others, so the element-wise int32 sum
+ * of every slab's d_state is the next round's input; a sample is marched by the slab holding its brick layer.  Stop
+ * when the summed hand-over count is 0; at most n_slabs rounds are needed.
+ * bslam_tsdf_raycast_shade: the outputs (as bslam_tsdf_raycast) of the finished rays whose trilinear base plane lies in
+ * this slab, 0 for every other pixel, from the summed final state: the int32 sum over the slabs is the full map.
+ * d_halo_lo / d_halo_hi: the neighbours' planes, packed as bslam_tsdf_raycast_halo_bytes(neighbour, planes) bytes:
+ * `planes` [nx][ny] float2 {tsdf, weight} planes, then (colour volumes) `planes` [nx][ny][3] f32 colour planes, then the
+ * [nby][nbx] brick flags of the brick layer that holds them.  d_halo_lo: 1 plane (z0 - 1) of the slab below, d_halo_hi:
+ * 2 planes (z1, z1 + 1) of the slab above; each is required exactly when that neighbour exists.  F = 0: NULL buffers are
+ * accepted and nothing is launched; any F (64 frames per launch). */
+BSLAM_API size_t bslam_tsdf_raycast_halo_bytes(const bslam_volume *vol, int planes);
+BSLAM_API int bslam_tsdf_raycast_segment(bslam_volume *vol, int n_slabs, const int *h_slab_z, int first, int F, int H, int W, const double *h_K,
+                                         const double *h_extrinsics, float depth_min, float depth_max, float weight_threshold, int32_t *d_state,
+                                         bslam_stream_t stream);
+BSLAM_API int bslam_tsdf_raycast_shade(bslam_volume *vol, int n_slabs, const int *h_slab_z, const void *d_halo_lo, const void *d_halo_hi, int F,
+                                       int H, int W, const double *h_K, const double *h_extrinsics, float depth_scale, const int32_t *d_state,
+                                       float *d_depth, float *d_vertex, float *d_normal, float *d_color, bslam_stream_t stream);
 /* bslam_vbg_raycast: tensor flavour (`MAP.synthesize_model_frame`) on a volume integrated by bslam_vbg_integrate with
  * the workspace d_vbg_workspace: 16^3 blocks on the world block grid, allocated = activated by any frame so far,
  * voxel-corner trilinear interpolation, sdf_trunc = trunc_voxel_multiplier * voxel_size, ray range from Open3D's
