@@ -24,6 +24,7 @@ def __getattr__(name):  # lazy: keep `import bodyslam_b200` light and torch-free
         "colorize": "mdem", "process_image": "mdem", "process_images": "mdem", "DepthEstimator": "mdem",
         "MDEMInterface": "mdem", "compute_median_scale_factor": "mdem",
         "ShardedTSDF": "sharding",
+        "RaycastingScene": "raycasting",
     }
     if name in table:
         return getattr(importlib.import_module(f"{__name__}.{table[name]}"), name)

@@ -84,6 +84,12 @@ _SIGNATURES = {
     "bslam_points_last_stats": (C.c_int, [_p, _p]),
     "bslam_points_count": (C.c_int, [_p, _p, _p]),
     "bslam_points_emit": (C.c_int, [_p, _p, _p, _p, _p, C.c_int64, _p]),
+    "bslam_mesh_bvh_bytes": (C.c_size_t, [C.c_int64]),
+    "bslam_mesh_build_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int]),
+    "bslam_mesh_build": (C.c_int, [_p, C.c_int64, _p, C.c_int64, _p, C.c_int, _p, _p, _p]),
+    "bslam_mesh_cast_rays": (C.c_int, [_p, _p, C.c_int64, _p, _p, _p, _p, _p, _p]),
+    "bslam_mesh_rays_pinhole": (C.c_int, [C.c_int, C.c_int, C.c_int, _p, _p, _p, _p]),
+    "bslam_mesh_cast_pinhole": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p, _p, _p, _p, _p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

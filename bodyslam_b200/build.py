@@ -14,7 +14,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libbodyslam_b200.so")
-SOURCES = ["bslam_tsdf.cu", "bslam_image.cu", "bslam_colorize_f32.cu", "bslam_extract.cu", "bslam_vbg.cu", "bslam_raycast.cu", "bslam_odometry.cu"]
+SOURCES = ["bslam_tsdf.cu", "bslam_image.cu", "bslam_colorize_f32.cu", "bslam_extract.cu", "bslam_vbg.cu", "bslam_raycast.cu", "bslam_odometry.cu",
+           "bslam_mesh_raycast.cu"]
 
 
 def nvcc_path() -> str:

@@ -439,6 +439,35 @@ BSLAM_API int bslam_odom_linearize(const float *d_frames, int F, const int *h_pa
                                    int method, float depth_outlier_trunc, float depth_huber_delta, float intensity_huber_delta, const double *h_T,
                                    double *d_sums, void *d_workspace, bslam_stream_t stream);
 
+/* ------------------------------------------------------------------ mesh ray casting
+ * Open3D's `t.geometry.RaycastingScene` (`cast_rays(...)["t_hit"]` as a synthetic depth map, N/3DM/
+ * synthetic_depth_generator.py:74-97): closest hits of rays against triangle meshes through an LBVH built on the device.
+ * The semantics are written down in the brute-force CPU reference tests/mesh_raycast_ref.c, which the GPU equals bit for
+ * bit; parity with Open3D / Embree is UNPINNED (DESIGN.md section 7, "Mesh ray cast exactness").
+ *
+ * bslam_mesh_build: d_verts [n_verts][3] f32 and d_tris [n_tris][3] i32 of every geometry, concatenated; h_geom
+ * [n_geoms + 1][2] i64 = {first triangle, first vertex} of each geometry, then {n_tris, n_verts}.  Triangle indices are
+ * local to their geometry.  d_bvh: bslam_mesh_bvh_bytes(n_tris) bytes, d_workspace: bslam_mesh_build_workspace_bytes(n_tris,
+ * n_geoms) bytes, both caller-owned; the workspace may be freed after the call's work has run.  Indices are validated on
+ * the device: the call synchronises the stream once to read the result and returns BSLAM_E_ARG with the geometry and
+ * triangle of the first index out of range.  Triangles with a non-finite coordinate or a zero float32 normal are left
+ * out of the scene.
+ *
+ * bslam_mesh_cast_rays: d_rays [n][6] f32 {origin, direction}; outputs [n]: t_hit (+inf on a miss), geometry and
+ * primitive ids (0xFFFFFFFF on a miss), optional d_uvs [n][2] (Embree's u, v) and d_normals [n][3] (unit, world frame),
+ * 0 on a miss.  bslam_mesh_rays_pinhole: the rays of F pinhole frames (h_K 3x3 row-major f64, h_extrinsics [F][16] f64
+ * world -> camera) into d_rays [F][H][W][6]; bslam_mesh_cast_pinhole: the same rays cast without storing them, outputs
+ * [F][H][W](...).  n == 0 or F * H * W == 0 launches nothing and accepts NULL buffers. */
+BSLAM_API size_t bslam_mesh_bvh_bytes(int64_t n_tris);
+BSLAM_API size_t bslam_mesh_build_workspace_bytes(int64_t n_tris, int n_geoms);
+BSLAM_API int bslam_mesh_build(const float *d_verts, int64_t n_verts, const int32_t *d_tris, int64_t n_tris, const int64_t *h_geom, int n_geoms,
+                               void *d_bvh, void *d_workspace, bslam_stream_t stream);
+BSLAM_API int bslam_mesh_cast_rays(const void *d_bvh, const float *d_rays, int64_t n, float *d_t_hit, uint32_t *d_geom_ids, uint32_t *d_prim_ids,
+                                   float *d_uvs, float *d_normals, bslam_stream_t stream);
+BSLAM_API int bslam_mesh_rays_pinhole(int F, int H, int W, const double *h_K, const double *h_extrinsics, float *d_rays, bslam_stream_t stream);
+BSLAM_API int bslam_mesh_cast_pinhole(const void *d_bvh, int F, int H, int W, const double *h_K, const double *h_extrinsics, float *d_t_hit,
+                                      uint32_t *d_geom_ids, uint32_t *d_prim_ids, float *d_uvs, float *d_normals, bslam_stream_t stream);
+
 /* Surface-extraction flavour of bslam_mc_* / bslam_points_*: a voxel is valid when weight >= weight_threshold
  * (0 = weight > 0, Open3D's legacy `weight != 0` for every weight an integrator writes: they differ only for negative
  * or NaN weights, which count as invalid here; the tensor pipeline's extract_triangle_mesh / extract_point_cloud default
