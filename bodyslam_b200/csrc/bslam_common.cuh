@@ -129,6 +129,8 @@ struct bslam_volume {
     int batch; // frames per integrate launch (0 = default)
     int prof_enabled, prof_n;
     int zpw;                                  // z layers per integrate warp (0 = auto by shard size)
+    void *rgb_tail;          // padded copy of a launch's last RGB frame (bslam_tsdf.cu: set_rgb_last)
+    size_t rgb_tail_bytes;
     // incremental point extraction (bslam_points_set_incremental): per-brick cache of the extracted points
     void *pts_cache;
     size_t pts_cache_bytes;

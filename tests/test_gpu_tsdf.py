@@ -54,7 +54,7 @@ def assert_volume_equal(vol, V, trunc, color=False):
     if color:
         c = out[2].cpu().numpy()
         ref = V.color.reshape(c.shape)
-        assert np.abs(c - ref).max() <= 1e-3
+        assert np.array_equal(c, ref), f"colour not bit-exact (max diff {np.abs(c - ref).max()})"
 
 
 @pytest.mark.parametrize("scene,res", [("laparoscopy512", 128), ("colonoscopy256", 64)])

@@ -1,7 +1,8 @@
 #!/bin/bash
 # compute-sanitizer over the hot path (run on a GPU box):  bash tools/sanitize.sh > gpurun_out/sanitizer.log
 # memcheck + racecheck + synccheck on smoke() (a4, K3 with named barriers / shared flag words / persistent
-# claims, K4 marching cubes, K1, K2) and on a small sharded-layout / unit-activation / colour integration.
+# claims, K4 marching cubes, K1, K2), on a small sharded-layout / unit-activation / colour integration and on colour
+# integrations whose RGB batches end exactly where their allocations do.
 set -u
 CS=/usr/local/cuda/bin/compute-sanitizer
 PY='
@@ -27,10 +28,19 @@ for kw in (dict(unit_activation=True), dict(gz0=8, z_total=64, z_interleave=2), 
         if "gz0" not in kw:
             v.extract_triangle_mesh(); v.extract_point_cloud()
 mdem.colorize(np.random.default_rng(0).uniform(0.1, 3, (120, 160)).astype(np.float32), cmap="viridis", invalid_val=0)
+# colour gathers at the end of the RGB batch (PYTORCH_NO_CUDA_MEMORY_CACHING=1 below: every tensor is its own exactly sized
+# cudaMalloc): the 512 x 512 x 144 laparoscopy slab (8 z layers per warp, no long-chain phase), then 3 frames of 333 x 201
+# px, whose RGB batch (200 799 pixels) ends 3 bytes short of a 4-byte word
+sl = small_scene("laparoscopy512", res=512, frames=2)
+v = DenseTSDFVolume(sl["voxel_length"], sl["sdf_trunc"], (512, 512, 144), sl["origin"], color=True, device=dev, gz0=368, z_total=512)
+v.integrate_batch(ops.depth_from_u16(sl["depth_u16"], 1000.0, 3.0, dev), torch.from_numpy(sl["color"]).to(dev), sl["intrinsic"], sl["E"])
+od = small_scene("laparoscopy512", res=64, frames=3, W=333, H=201)
+v = DenseTSDFVolume(od["voxel_length"], od["sdf_trunc"], 64, od["origin"], color=True, device=dev)
+v.integrate_batch(ops.depth_from_u16(od["depth_u16"], 1000.0, 3.0, dev), torch.from_numpy(od["color"]).to(dev), od["intrinsic"], od["E"])
 torch.cuda.synchronize()
 print("SANITIZE_WORKLOAD_OK")
 '
 for tool in memcheck racecheck synccheck; do
   echo "=== compute-sanitizer --tool $tool"
-  timeout 900 $CS --tool $tool --print-limit 20 python -c "$PY" 2>&1 | grep -E "SANITIZE_WORKLOAD_OK|smoke ok|ERROR SUMMARY|RACECHECK SUMMARY|Race reported|Invalid|hazard|error" | head -40
+  PYTORCH_NO_CUDA_MEMORY_CACHING=1 timeout 900 $CS --tool $tool --print-limit 20 python -c "$PY" 2>&1 | grep -E "SANITIZE_WORKLOAD_OK|smoke ok|ERROR SUMMARY|RACECHECK SUMMARY|Race reported|Invalid|hazard|error" | head -40
 done
