@@ -13,6 +13,7 @@ _lib = None
 OK, E_ARG, E_CUDA, E_CAPACITY = 0, -1, -2, -3
 MAX_BATCH = 256
 ZMARCH_BRICK, ZMARCH_LITERAL = 8, 0
+GROW_OK, GROW_GROWN, GROW_CAP_UNITS, GROW_CAP_ROW_WORDS = 0, 1, 2, 3
 
 _p = C.c_void_p
 _SIGNATURES = {
@@ -37,6 +38,8 @@ _SIGNATURES = {
     "bslam_tsdf_destroy": (C.c_int, [_p]),
     "bslam_tsdf_reset": (C.c_int, [_p, _p]),
     "bslam_tsdf_copy": (C.c_int, [_p, _p, _p]),
+    "bslam_tsdf_unit_bounds": (C.c_int, [_p, _p, C.c_int, C.c_float, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p, _p]),
+    "bslam_tsdf_grow_box": (C.c_int, [_p, _p, _p, _p, _p, _p]),
     "bslam_tsdf_integrate": (C.c_int, [_p, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, C.c_int, _p, C.c_int, _p]),
     "bslam_tsdf_integrate_u16": (C.c_int, [_p, _p, C.c_float, C.c_float, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p]),
     "bslam_tsdf_prepare_u16": (C.c_int, [_p, _p, C.c_float, C.c_float, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p]),

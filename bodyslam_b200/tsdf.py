@@ -70,6 +70,9 @@ class DenseTSDFVolume:
             _lib.check(self._L.bslam_tsdf_set_unit_activation(self._h, int(unit_resolution), -1, int(self.z_total)))
             self.unit_resolution, self.depth_sampling_stride = int(unit_resolution), -1
         self.frames_integrated = 0
+        self._auto_grow = False
+        self.grow_capped = None      # after a growth refused by a unit cap: which cap (see set_auto_grow)
+        self.growth_events = 0
 
     def set_unit_activation(self, unit_resolution: int = 32, depth_sampling_stride: int = 8):
         """ScalableTSDFVolume semantics (what the reference's `TSDF()` builds, tsdf.py:7-12): a frame
@@ -121,6 +124,7 @@ class DenseTSDFVolume:
         with torch.cuda.device(self.device):
             _lib.check(self._L.bslam_tsdf_copy(self._h, other._h, _lib.stream_ptr(self.device)))
         other.frames_integrated = self.frames_integrated
+        other._auto_grow = self._auto_grow
         return other
 
     def reset(self):
@@ -176,6 +180,8 @@ class DenseTSDFVolume:
         E = np.ascontiguousarray(np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 16))
         if E.shape[0] != F:
             raise RuntimeError(f"integrate_batch: {F} frames but {E.shape[0]} extrinsics")
+        if self._auto_grow and not dry_run:
+            self._grow_for(self.unit_bounds(depth, intrinsic, E))
         K = np.array([fx, fy, cx, cy], dtype=np.float64)
         with torch.cuda.device(self.device):
             _lib.check(self._L.bslam_tsdf_integrate(self._h, _lib.ptr(depth), _lib.ptr(color) if self.color else None, F, H, W,
@@ -202,6 +208,7 @@ class DenseTSDFVolume:
             raise RuntimeError(f"integrate_u16_batch: {F} frames but {E.shape[0]} extrinsics")
         if scratch is None or scratch.numel() < F * H * W:
             scratch = torch.empty((F, H, W), dtype=torch.float32, device=self.device)
+        self._auto_grow_u16(depth_u16, intrinsic, E, depth_scale, depth_trunc)
         K = np.array([fx, fy, cx, cy], dtype=np.float64)
         with torch.cuda.device(self.device):
             _lib.check(self._L.bslam_tsdf_integrate_u16(self._h, _lib.ptr(depth_u16), float(depth_scale), float(depth_trunc or 0.0),
@@ -225,10 +232,19 @@ class DenseTSDFVolume:
             self._copy_stream = torch.cuda.Stream(self.device)
         return self._copy_stream
 
+    def _refuse_split_halves(self, name):
+        if self._auto_grow:
+            raise RuntimeError(f"{name}: the prepared state lives in the volume's handle, which growth replaces; "
+                               "an auto-growing volume integrates through integrate_host / integrate_u16_chunks / integrate_u16_batch")
+
     def prepare_u16(self, depth_u16, intrinsic, extrinsics, scratch, depth_scale: float = 1000.0, depth_trunc: float = 3.0, wait=None):
         """enqueue the preparation of one launch (<= 256 frames; see bslam_tsdf_prepare_u16) on the side stream.
         `wait`: optional callable run with the side stream current (e.g. `work.wait` of an NCCL transfer or
         `lambda: stream.wait_event(ev)`) -- what the frames' arrival is ordered by.  Up to two launches ahead."""
+        self._refuse_split_halves("prepare_u16")
+        self._prepare_u16(depth_u16, intrinsic, extrinsics, scratch, depth_scale, depth_trunc, wait)
+
+    def _prepare_u16(self, depth_u16, intrinsic, extrinsics, scratch, depth_scale, depth_trunc, wait):
         torch = _lib.require_cuda()
         W, H, fx, fy, cx, cy = intrinsic_params(intrinsic)
         if depth_u16.dim() == 2:
@@ -254,6 +270,10 @@ class DenseTSDFVolume:
 
     def integrate_prepared(self, color=None, update_counts=None):
         """enqueue the integration of the oldest prepared launch on the current stream"""
+        self._refuse_split_halves("integrate_prepared")
+        self._integrate_prepared(color, update_counts)
+
+    def _integrate_prepared(self, color, update_counts):
         torch = _lib.require_cuda()
         F, _, _ = self._prepared.pop(0)
         if self.color and color is None:
@@ -273,6 +293,10 @@ class DenseTSDFVolume:
         staging buffers chunk k may use (the f32 one always receives its converted frames), `free` is the event after
         which the current stream no longer reads them.  It returns the chunk's uint16 frames on the device, its colour
         (or None) and the callable the side stream runs before the preparation (or None)."""
+        self._refuse_split_halves("integrate_streamed")
+        self._integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts, color_staging)
+
+    def _integrate_streamed(self, chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts, color_staging=False):
         torch = _lib.require_cuda()
         if not chunks:
             return
@@ -287,7 +311,7 @@ class DenseTSDFVolume:
 
             def prep(k):
                 f0, f1 = chunks[k]
-                self.prepare_u16(arrived[k][0], intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc, wait=arrived[k][2])
+                self._prepare_u16(arrived[k][0], intrinsic, E[f0:f1], stage[k % 3][1], depth_scale, depth_trunc, arrived[k][2])
 
             for k in range(min(2, len(chunks))):
                 arrived[k] = arrive(k, stage[k % 3], free[k % 3])
@@ -297,7 +321,7 @@ class DenseTSDFVolume:
                     arrived[k + 2] = arrive(k + 2, stage[(k + 2) % 3], free[(k + 2) % 3])
                 if k + 1 < len(chunks):
                     prep(k + 1)
-                self.integrate_prepared(arrived.pop(k)[1], None if update_counts is None else update_counts[f0:f1])
+                self._integrate_prepared(arrived.pop(k)[1], None if update_counts is None else update_counts[f0:f1])
                 free[k % 3] = torch.cuda.Event()
                 free[k % 3].record(main)
 
@@ -310,7 +334,10 @@ class DenseTSDFVolume:
             f0, f1 = chunks[k]
             return depth_u16[f0:f1], None if color is None else color[f0:f1], None
 
-        self.integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts)
+        if self._auto_grow and chunks:
+            a, b = chunks[0][0], chunks[-1][1]
+            self._auto_grow_u16(depth_u16[a:b], intrinsic, np.asarray(to_numpy(extrinsics)).reshape(-1, 16)[a:b], depth_scale, depth_trunc)
+        self._integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts)
 
     @staticmethod
     def stream_chunks(F: int, chunk: int = 256, ramp=(32, 64, 128), multiple_of: int = 1):
@@ -377,6 +404,10 @@ class DenseTSDFVolume:
         if self.color and color is None:
             raise RuntimeError("[DenseTSDFVolume::IntegrateHost] Unsupported image format.")
         chunks = self.stream_chunks(depth_u16.shape[0], chunk)
+        if self._auto_grow and chunks:
+            # bounds pass on the stride-sampled pixels only (1/64 of the depth bytes at stride 8), gathered on the host
+            s = self.depth_sampling_stride
+            self._auto_grow_u16(depth_u16[:, ::s, ::s].contiguous().to(self.device), intrinsic, extrinsics, depth_scale, depth_trunc, sampled=True)
         cs = self.copy_stream()
 
         def arrive(k, stage, free):      # H2D of chunk k on the copy stream, once the current stream is done with its buffers
@@ -391,7 +422,7 @@ class DenseTSDFVolume:
                 copied.record(cs)
             return u16[:f1 - f0], col[:f1 - f0] if use_color else None, copied.wait
 
-        self.integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts, use_color)
+        self._integrate_streamed(chunks, intrinsic, extrinsics, arrive, depth_scale, depth_trunc, update_counts, use_color)
 
     def count_updates(self, depth, intrinsic, extrinsics, zmarch: int = _lib.ZMARCH_BRICK):
         """U_f of SURVEY.md 8(d): voxels each frame WOULD update (volume untouched) -> i64 [F]."""
@@ -422,14 +453,17 @@ class DenseTSDFVolume:
     def set_z_split(self, z_layers_per_warp: int):
         """z layers per integrate warp: 8, 4, 2 or 0 = automatic (see bslam_tsdf_set_z_split)"""
         _lib.check(self._L.bslam_tsdf_set_z_split(self._h, int(z_layers_per_warp)))
+        self._z_split = int(z_layers_per_warp)
 
     def set_batch(self, frames_per_launch: int):
         """frames per integrate launch (0 = library default, max 256)"""
         _lib.check(self._L.bslam_tsdf_set_batch(self._h, int(frames_per_launch)))
+        self._batch = int(frames_per_launch)
 
     def profile(self, enable: bool = True):
         """bracket the dominant integrate kernel with CUDA events (bench.py roofline)"""
         _lib.check(self._L.bslam_tsdf_profile(self._h, int(bool(enable))))
+        self._profiling = bool(enable)
 
     def profile_read(self):
         """-> (accumulated kernel ms, launches) since profile(True); synchronises"""
@@ -447,6 +481,7 @@ class DenseTSDFVolume:
         """dense mode: count the stride-sampled depth points of every integrated frame that fall outside the
         box (unit-activation mode always does); 0 = off.  See `clip_stats`."""
         _lib.check(self._L.bslam_tsdf_set_clip_check(self._h, int(sampling_stride), int(self.z_total)))
+        self._clip_check = int(sampling_stride)
 
     def clip_stats(self, reset: bool = False):
         """The reference's volume is unbounded, this box is not: -> dict(points, outside, partly_outside) over the
@@ -454,6 +489,127 @@ class DenseTSDFVolume:
         out = (C.c_ulonglong * 3)()
         _lib.check(self._L.bslam_tsdf_clip_stats(self._h, out, int(bool(reset)), _lib.stream_ptr(self.device)))
         return {"points": int(out[0]), "outside": int(out[1]), "partly_outside": int(out[2])}
+
+    # ------------------------------------------------------------------ growth (unit-activation mode)
+    def set_auto_grow(self, enable: bool = True):
+        """Grow the box with the scene, like the reference's unbounded ScalableTSDFVolume: every integrate call first runs
+        one bounds pass over all of its frames (`unit_bounds`) and, when they activate units outside the box, grows it
+        once (`grow_to`, policy of bslam_tsdf_grow_box) before integrating.  A box grown by whole units on the world unit
+        grid integrates exactly like one that was that large from the start.  When the box needed breaks a unit cap it
+        stays as it is, the points outside it are clipped and counted (`clip_stats`), and `grow_capped` names the cap.
+        Needs unit-activation mode on a whole (not z-sharded) box; the split `prepare_u16` / `integrate_prepared` /
+        `integrate_streamed` halves refuse an auto-growing volume."""
+        if enable and not (self.unit_activation and self.gz0 == 0 and self.z_total == self.nz and self.z_interleave == 1):
+            raise RuntimeError("set_auto_grow: growth needs a whole box in unit-activation mode (not the dense rule, unit_arithmetic "
+                               "or a z-shard view)")
+        self._auto_grow = bool(enable)
+
+    def _unit_geometry(self):
+        ul = self.voxel_length * self.unit_resolution
+        u0 = np.rint(self.origin / ul).astype(np.int64)
+        nu = np.array([self.nx, self.ny, self.nz], dtype=np.int64) // self.unit_resolution
+        return ul, u0, nu
+
+    def unit_bounds(self, depth, intrinsic, extrinsics, depth_scale: float = 1000.0, depth_trunc: float = 3.0, sampled: bool = False):
+        """[[lo x, y, z], [hi x, y, z]] (int64) GLOBAL unit indices of the units that these frames would activate (see
+        bslam_tsdf_unit_bounds), or None when no pixel gives a point.  depth: [F,H,W] f32 metres or uint16 (converted
+        with depth_scale / depth_trunc like `integrate_u16_batch`) on the device; sampled=True: only the stride-sampled
+        pixels, [F, ceil(H / stride), ceil(W / stride)].  Synchronises."""
+        torch = _lib.require_cuda()
+        W, H, fx, fy, cx, cy = intrinsic_params(intrinsic)
+        u16 = ops._dtype_name(depth) == "uint16"
+        d = ops.as_cuda(depth, torch.uint16 if u16 else torch.float32, self.device).contiguous()
+        E = np.ascontiguousarray(np.asarray(to_numpy(extrinsics), dtype=np.float64).reshape(-1, 16))
+        s = getattr(self, "depth_sampling_stride", 8)
+        hw = ((H + s - 1) // s, (W + s - 1) // s) if sampled else (H, W)
+        if d.dim() == 2:
+            d = d.unsqueeze(0)
+        if d.dim() != 3 or tuple(d.shape[1:]) != hw or d.shape[0] != E.shape[0]:
+            raise RuntimeError(f"unit_bounds: depth of shape {tuple(d.shape)} for {E.shape[0]} poses of {H}x{W} images (sampled={sampled})")
+        K = np.array([fx, fy, cx, cy], dtype=np.float64)
+        out = np.zeros(6, np.int64)
+        valid = C.c_int()
+        with torch.cuda.device(self.device):
+            _lib.check(self._L.bslam_tsdf_unit_bounds(self._h, _lib.ptr(d), int(u16), float(depth_scale), float(depth_trunc or 0.0), E.shape[0], H, W,
+                                                      int(bool(sampled)), _lib.ptr(K), _lib.ptr(E), _lib.ptr(out), C.byref(valid),
+                                                      _lib.stream_ptr(self.device)))
+        return out.reshape(2, 3) if valid.value else None
+
+    def _grow_for(self, bounds):
+        """grow (at most once) so that the box holds the units `bounds`; -> True when it grew"""
+        if bounds is None:
+            return False
+        ul, u0, nu = self._unit_geometry()
+        req = np.ascontiguousarray(np.asarray(bounds, dtype=np.int64).reshape(6))
+        new_u0, new_nu, status = np.zeros(3, np.int64), np.zeros(3, np.int64), C.c_int()
+        _lib.check(self._L.bslam_tsdf_grow_box(_lib.ptr(u0), _lib.ptr(nu), _lib.ptr(req), _lib.ptr(new_u0), _lib.ptr(new_nu), C.byref(status)))
+        if status.value == _lib.GROW_GROWN:
+            return self.grow_to(new_u0 * ul, new_nu * self.unit_resolution)
+        if status.value != _lib.GROW_OK:
+            self.grow_capped = ("65 536 units (or unit indices beyond +-2^30)" if status.value == _lib.GROW_CAP_UNITS
+                                else "nux * nuy * ceil(nuz / 32) <= 4096 units")
+        return False
+
+    def _auto_grow_u16(self, depth_u16, intrinsic, extrinsics, depth_scale, depth_trunc, sampled=False):
+        if self._auto_grow:
+            self._grow_for(self.unit_bounds(depth_u16, intrinsic, extrinsics, depth_scale, depth_trunc, sampled))
+
+    def grow_to(self, origin, resolution) -> bool:
+        """Grow the box IN PLACE to `resolution` voxels from corner `origin`, a larger box on the same brick grid that
+        contains this one (whole units on the world unit grid in unit-activation mode): new storage, the contents
+        relocated (bslam_tsdf_copy), every setting re-applied, `frames_integrated` kept.  The point cache of incremental
+        extraction starts over (same output).  Peak device memory: both boxes.  When the new box cannot be allocated
+        the old one stays and a warning is issued once; -> False."""
+        import warnings
+
+        torch = _lib.require_cuda()
+        if getattr(self, "_prepared", None):
+            raise RuntimeError("grow_to: a prepared launch is pending")
+        if self.gz0 != 0 or self.z_total != self.nz or self.z_interleave != 1:
+            raise RuntimeError("grow_to: z-shard views cannot grow")
+        res = (int(resolution),) * 3 if np.isscalar(resolution) else tuple(int(r) for r in resolution)
+        origin = np.ascontiguousarray(origin, dtype=np.float64)
+        if res == (self.nx, self.ny, self.nz):
+            if np.array_equal(origin, self.origin):
+                return False
+            raise RuntimeError("grow_to: a box of the same size must stay where it is")
+        h = C.c_void_p()
+        try:
+            storage = torch.empty(self._L.bslam_tsdf_storage_bytes(*res, int(self.color)), dtype=torch.uint8, device=self.device)
+            with torch.cuda.device(self.device):
+                _lib.check(self._L.bslam_tsdf_create(C.byref(h), *res, 0, self.voxel_length, self.sdf_trunc, _lib.ptr(origin), int(self.color),
+                                                     self.device.index, _lib.ptr(storage), _lib.stream_ptr(self.device)))
+        except (torch.OutOfMemoryError, RuntimeError) as e:
+            if h.value:
+                self._L.bslam_tsdf_destroy(h)
+            if "out of memory" not in str(e).lower() and "cudamalloc" not in str(e).lower():
+                raise
+            if not getattr(self, "_grow_oom_warned", False):
+                self._grow_oom_warned = True
+                warnings.warn(f"DenseTSDFVolume.grow_to: cannot allocate a {res[0]}x{res[1]}x{res[2]} box ({e}); the box stays "
+                              f"{self.nx}x{self.ny}x{self.nz} and points outside it are clipped")
+            return False
+        with torch.cuda.device(self.device):
+            rc = self._L.bslam_tsdf_copy(self._h, h, _lib.stream_ptr(self.device))
+            if rc != _lib.OK:
+                self._L.bslam_tsdf_destroy(h)
+                _lib.check(rc)
+            self._storage.record_stream(torch.cuda.current_stream(self.device))
+            self._L.bslam_tsdf_destroy(self._h)
+        self._h, self._storage = h, storage
+        self.nx, self.ny, self.nz = res
+        self.z_total = self.nz
+        self.origin = origin
+        if self.unit_activation:
+            self.set_unit_activation(self.unit_resolution, self.depth_sampling_stride)
+        if getattr(self, "_pts_incremental", False):
+            self.set_incremental_points(True, self._pts_inc_normals)
+        for attr, fn in (("_z_split", self.set_z_split), ("_batch", self.set_batch), ("_clip_check", self.set_clip_check),
+                         ("_profiling", self.profile)):
+            if hasattr(self, attr):
+                fn(getattr(self, attr))
+        self.growth_events += 1
+        return True
 
     # ------------------------------------------------------------------ dense views (parity / interchange)
     def export_dense(self, with_color: bool = False):
@@ -648,7 +804,7 @@ class TSDF:
     """Drop-in for the reference's `TSDF` (N/3DM/tsdf.py:5-52)."""
 
     def __init__(self, voxel_length: float = 0.001, sdf_trunc: float = 0.1, resolution=512, origin=None,
-                 color: bool = True, device=None, unit_activation=None):
+                 color: bool = True, device=None, unit_activation=None, grow: bool = False):
         """unit_activation: True = ScalableTSDFVolume semantics (volume_unit_resolution 32, depth_sampling_stride
         8, tsdf.py:11-12): a frame only integrates the 32^3 units its sampled depth points activate, exactly
         what the reference object does; False = every voxel of the box follows the UniformTSDFVolume rule
@@ -659,7 +815,11 @@ class TSDF:
         is RE-CENTRED ON THE FIRST FRAME's back-projected depth points (snapped to the 32-voxel unit grid) when that
         frame would otherwise mostly fall outside it -- the reference's hashed volume is unbounded, and its SLAM
         loop starts at the identity pose looking down +z (N/3DM/slam.py), i.e. at a surface that lies in front of,
-        not around, the origin."""
+        not around, the origin.
+
+        grow: the box grows with the scene (`DenseTSDFVolume.set_auto_grow`): every frame's activated units are kept, as
+        by the reference's unbounded volume, bit for bit what a box sized for the whole trajectory holds.  Needs
+        unit-activation mode; points are only dropped (and warned about) once a growth would break a unit cap."""
         res = (int(resolution),) * 3 if np.isscalar(resolution) else tuple(int(r) for r in resolution)
         org = origin if origin is not None else tuple(-0.5 * r * voxel_length for r in res)
         self._auto_origin = origin is None
@@ -668,10 +828,10 @@ class TSDF:
                                                    color=color, device=device, unit_activation=ua)
         if unit_activation is None:
             unit_activation = DenseTSDFVolume.unit_aligned(res, voxel_length, org)
-        self.tsdf = self._make(origin, bool(unit_activation))
-        if not unit_activation:
-            self.tsdf.set_clip_check(8)
-        self.tsdf.set_incremental_points(True, normals=True)      # extract_pcd() runs after every frame in the reference's loop
+        self._grow = bool(grow)
+        if self._grow and not unit_activation:
+            raise RuntimeError("TSDF(grow=True) needs unit activation: a box of whole 32^3 units on the world unit grid")
+        self._setup(self._make(origin, bool(unit_activation)), bool(unit_activation))
         self._clip_warned = 0.0
         self._next_clip_check = 1      # frames_integrated at which the next (synchronising) clip check is due
 
@@ -703,14 +863,19 @@ class TSDF:
         ua = self._unit_request
         if ua is None:
             ua = DenseTSDFVolume.unit_aligned((v.nx, v.ny, v.nz), v.voxel_length, new_origin)
-        self.tsdf = self._make(tuple(new_origin), bool(ua))
-        if not ua:
-            self.tsdf.set_clip_check(8)
-        self.tsdf.set_incremental_points(True, normals=True)
+        self._setup(self._make(tuple(new_origin), bool(ua)), bool(ua))
         warnings.warn(f"TSDF: only {100 * inside:.0f} % of the first frame's depth points fell inside the default box around the world "
                       f"origin; the box was re-centred on them: origin = ({new_origin[0]:.3f}, {new_origin[1]:.3f}, {new_origin[2]:.3f}) m, "
                       f"edge {ext[0]:.3f} m (pass origin= / resolution= to TSDF() to choose the box yourself)")
         return True
+
+    def _setup(self, vol, unit_activation):
+        self.tsdf = vol
+        if not unit_activation:
+            vol.set_clip_check(8)
+        vol.set_incremental_points(True, normals=True)      # extract_pcd() runs after every frame in the reference's loop
+        if self._grow:
+            vol.set_auto_grow(True)
 
     def clipped_fraction(self) -> float:
         """share of the sampled depth points integrated so far that fell OUTSIDE the bounded box (the
@@ -723,7 +888,7 @@ class TSDF:
 
         # the counters live on the device: read them at frames 1, 4, 16, ... so the per-frame cadence
         # (extract_pcd after every build_3D_map, N/3DM/slam.py:195) does not pay a device round trip per call
-        if self.tsdf.frames_integrated < self._next_clip_check:
+        if self.tsdf.frames_integrated < self._next_clip_check or (self._grow and self.tsdf.grow_capped is None):
             return
         while self._next_clip_check <= self.tsdf.frames_integrated:
             self._next_clip_check *= 4
@@ -734,7 +899,9 @@ class TSDF:
             hi = lo + np.array([self.tsdf.nx, self.tsdf.ny, self.tsdf.z_total]) * self.tsdf.voxel_length
             warnings.warn(f"TSDF: {100 * frac:.1f} % of the depth points integrated so far lie outside the volume box "
                           f"[{lo[0]:.3f}, {hi[0]:.3f}] x [{lo[1]:.3f}, {hi[1]:.3f}] x [{lo[2]:.3f}, {hi[2]:.3f}] m and were dropped "
-                          f"(the reference's ScalableTSDFVolume is unbounded); pass resolution= / origin= to TSDF() to cover the scene")
+                          f"(the reference's ScalableTSDFVolume is unbounded); " +
+                          (f"the box could not grow further: the unit cap of {self.tsdf.grow_capped}" if self._grow else
+                           "pass resolution= / origin= (or grow=True) to TSDF() to cover the scene"))
 
     def build_3D_map(self, rgbd, intrinsic, extrinsic):
         '''

@@ -161,8 +161,38 @@ BSLAM_API int bslam_tsdf_create(bslam_volume **out, int nx, int ny, int nz, int 
                                 int with_color, int device, void *d_storage, bslam_stream_t stream);
 BSLAM_API int bslam_tsdf_destroy(bslam_volume *vol);
 BSLAM_API int bslam_tsdf_reset(bslam_volume *vol, bslam_stream_t stream);
-/* deepcopy of N/3DM/tsdf.py:24 (build_copy_3D_map): dst must have identical geometry */
+/* deepcopy of N/3DM/tsdf.py:24 (build_copy_3D_map) when dst has src's geometry (one device-to-device copy).
+ * Relocation (box growth): dst may also be a LARGER box on the same device and brick grid that contains src -- same
+ * voxel_length, sdf_trunc and colour, dims multiples of 8, no z-shard, origins a whole number of bricks apart.  One kernel
+ * then writes every byte of dst once: src's voxels, colours and brick flags at that brick offset, what bslam_tsdf_reset
+ * writes everywhere else; src's out-of-box point counters (bslam_tsdf_clip_stats) carry over.  Any other geometry is a
+ * BSLAM_E_ARG "geometry mismatch". */
 BSLAM_API int bslam_tsdf_copy(const bslam_volume *src, bslam_volume *dst, bslam_stream_t stream);
+
+/* ------------------------------------------------------------------ box growth (unit-activation mode)
+ * bslam_tsdf_unit_bounds: min / max GLOBAL unit index per axis (h_bounds6 = lo x, y, z, hi x, y, z) of the units that F
+ * frames would activate -- the same stride-sampled pixels, f64 back-projection, pose product and
+ * floor((w -+ sdf_trunc) / unit_len) as the activation pass of the integration, whatever the box.  Points whose world
+ * coordinate is not finite are skipped; indices are clamped to +-2^40 (far beyond the caps) instead of wrapping.
+ * d_depth: f32 metres, or (depth_is_u16) uint16 converted like bslam_tsdf_integrate_u16 (f32(u) / depth_scale,
+ * >= depth_trunc -> 0 when depth_trunc > 0).  sampled = 1: the frames hold only the sampled pixels,
+ * [F][ceil(H / stride)][ceil(W / stride)] (H, W stay the full image size).  *h_valid = 0 when no pixel gave a point.
+ * Needs unit-activation mode; synchronises the stream.
+ * bslam_tsdf_grow_box: the growth policy.  Box of h_nu units from global unit h_u0 per axis; request h_bounds6 (as
+ * above; lo > hi on an axis = nothing requested).  The new box is the smallest one that holds the old box and the
+ * requested units, each side that had to move extended by a quarter of the old extent on its axis (>= 1 unit) unless
+ * that slack would break a cap.  *h_status: BSLAM_GROW_OK (the box already holds the request: unchanged),
+ * BSLAM_GROW_GROWN, or the cap that the smallest box breaks (unchanged): BSLAM_GROW_CAP_UNITS (65 536 units, or unit
+ * indices beyond +-2^30), BSLAM_GROW_CAP_ROW_WORDS (nux * nuy * ceil(nuz / 32) <= 4096).  Host only. */
+#define BSLAM_GROW_OK 0
+#define BSLAM_GROW_GROWN 1
+#define BSLAM_GROW_CAP_UNITS 2
+#define BSLAM_GROW_CAP_ROW_WORDS 3
+BSLAM_API int bslam_tsdf_unit_bounds(bslam_volume *vol, const void *d_depth, int depth_is_u16, float depth_scale, float depth_trunc,
+                                     int F, int H, int W, int sampled, const double *h_K, const double *h_extrinsics,
+                                     long long *h_bounds6, int *h_valid, bslam_stream_t stream);
+BSLAM_API int bslam_tsdf_grow_box(const long long *h_u0, const long long *h_nu, const long long *h_bounds6,
+                                  long long *h_new_u0, long long *h_new_nu, int *h_status);
 
 /*
  * Replaces `TSDF.build_3D_map(rgbd, intrinsic, extrinsic)` N/3DM/tsdf.py:14-22 (Open3D
