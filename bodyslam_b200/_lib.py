@@ -93,6 +93,12 @@ _SIGNATURES = {
     "bslam_mesh_cast_rays": (C.c_int, [_p, _p, C.c_int64, _p, _p, _p, _p, _p, _p]),
     "bslam_mesh_rays_pinhole": (C.c_int, [C.c_int, C.c_int, C.c_int, _p, _p, _p, _p]),
     "bslam_mesh_cast_pinhole": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "bslam_mesh_closest_points": (C.c_int, [_p, _p, C.c_int64, _p, _p, _p, _p, _p, _p]),
+    "bslam_mesh_distance": (C.c_int, [_p, _p, C.c_int64, _p, _p]),
+    "bslam_mesh_occupancy": (C.c_int, [_p, _p, C.c_int64, C.c_int, _p, _p, _p]),
+    "bslam_mesh_count_intersections": (C.c_int, [_p, _p, C.c_int64, _p, _p]),
+    "bslam_mesh_test_occlusions": (C.c_int, [_p, _p, C.c_int64, C.c_float, C.c_float, _p, _p]),
+    "bslam_mesh_occupancy_directions": (C.c_int, [C.c_int, _p]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

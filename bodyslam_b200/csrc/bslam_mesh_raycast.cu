@@ -306,6 +306,310 @@ __global__ void __launch_bounds__(256) mesh_rays_pinhole_kernel(const __grid_con
     for (int k = 0; k < 6; ++k) rays[6 * i + k] = r[k];
 }
 
+// ------------------------------------------------------------------ point and ray queries
+// Closest points (Open3D's compute_closest_points / compute_distance), intersection counts, occlusion and occupancy /
+// signed distance, equal bit for bit to the brute force of tests/mesh_query_ref.c whatever the traversal order.
+//
+// Counts and occlusion have no best t to prune by: a node is pruned only if its interval [a, b] is empty (a > b: the
+// ray misses the box) or misses [tnear, tfar] ([0, +inf) for counts), and a hit counts only if mr_tri_hit accepts it
+// and tnear <= t <= tfar.  By the containment property of mr_box_interval (an accepted t lies in the interval of the
+// triangle's own box, which lies in the interval of every node above it), a node above an accepted hit has
+// a <= t <= b, a <= tfar and b >= tnear, so it is never pruned and every accepted hit is reached (a NaN a prunes
+// nothing).  Occlusion may stop at the first one.  Without the a > b test a ray with tfar = +inf would visit nearly
+// every box ahead of its origin, since a box it misses has a finite b >= 0.
+//
+// Closest point: lb(box, q) = (g_0^2 + g_1^2) + g_2^2 with g_k = max(lo_k - q_k, q_k - hi_k, 0) in float32.  Each step
+// is monotone in the box, rounding included (a smaller lo or a larger hi never increases g_k, squares and sums of
+// non-negative values are monotone), and node boxes are exact min / max unions, so lb(node) <= lb(child) <= lb(own box of
+// any triangle below).  The computed d^2 of a triangle can round below its own box's bound, so triangles are ranked by
+// key = max(d^2, lb(own box)) >= lb(node above), in the reference too, and the result is the lexicographic minimum of
+// (key, g, p).  A node is pruned iff lb(node) > key_best: the final winner W has key_W <= key_best at every moment, hence
+// lb(node above W) <= key_W <= key_best and W is reached.  The comparison is strict so that a triangle whose key ties the
+// best, and which may win on a smaller (g, p), is still reached.  d^2 and lb are never NaN (differences of finite values
+// square to [0, +inf]), and a key of +inf (far or huge coordinates) prunes nothing.
+
+#include "bslam_mesh_dirs.h"
+
+struct MrDirs {
+    int n;
+    float d[BSLAM_MESH_MAX_SAMPLES][3];
+};
+
+__host__ __device__ __forceinline__ float mr_dot(const float a[3], const float b[3]) { return (a[0] * b[0] + a[1] * b[1]) + a[2] * b[2]; }
+
+// lower bound of the squared distance from q to the box [lo, hi]
+__host__ __device__ __forceinline__ float mr_box_lb(const float lo[3], const float hi[3], const float q[3]) {
+    float g[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const float a = lo[k] - q[k], b = q[k] - hi[k];
+        const float m = b > a ? b : a;
+        g[k] = m > 0.0f ? m : 0.0f;
+    }
+    return (g[0] * g[0] + g[1] * g[1]) + g[2] * g[2];
+}
+
+// Ericson, Real-Time Collision Detection 5.1.5 (ClosestPtPointTriangle) in float32: the closest point c of triangle v to
+// p with its weights u (of v1) and w (of v2).  When a region's division fails (0 / 0, an overflow) and c or (u, w) is
+// not finite, the triangle's nearest vertex stands in (the first of v0, v1, v2 on a tie of d^2).  -> d^2 = |c - p|^2
+__host__ __device__ __forceinline__ float mr_closest_tri(const float p[3], const float v[9], float c[3], float &u, float &w) {
+    const float *a = v, *b = v + 3, *cc = v + 6;
+    float ab[3], ac[3], ap[3], bp[3], cp[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) { ab[k] = b[k] - a[k]; ac[k] = cc[k] - a[k]; ap[k] = p[k] - a[k]; bp[k] = p[k] - b[k]; cp[k] = p[k] - cc[k]; }
+    const float d1 = mr_dot(ab, ap), d2 = mr_dot(ac, ap), d3 = mr_dot(ab, bp), d4 = mr_dot(ac, bp), d5 = mr_dot(ab, cp), d6 = mr_dot(ac, cp);
+    const float vc = d1 * d4 - d3 * d2, vb = d5 * d2 - d1 * d6, va = d3 * d6 - d5 * d4;
+    int region;
+    float s = 0.0f, t = 0.0f;
+    if (d1 <= 0.0f && d2 <= 0.0f) region = 0;                                        // vertex v0
+    else if (d3 >= 0.0f && d4 <= d3) region = 1;                                     // vertex v1
+    else if (vc <= 0.0f && d1 >= 0.0f && d3 <= 0.0f) { region = 3; s = d1 / (d1 - d3); }              // edge v0 v1
+    else if (d6 >= 0.0f && d5 <= d6) region = 2;                                     // vertex v2
+    else if (vb <= 0.0f && d2 >= 0.0f && d6 <= 0.0f) { region = 4; t = d2 / (d2 - d6); }             // edge v0 v2
+    else if (va <= 0.0f && (d4 - d3) >= 0.0f && (d5 - d6) >= 0.0f) {                 // edge v1 v2
+        region = 5;
+        t = (d4 - d3) / ((d4 - d3) + (d5 - d6));
+    } else {                                                                         // face
+        region = 6;
+        const float den = 1.0f / ((va + vb) + vc);
+        s = vb * den;
+        t = vc * den;
+    }
+    bool ok = true;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        float x;
+        if (region == 0) x = a[k];
+        else if (region == 1) x = b[k];
+        else if (region == 2) x = cc[k];
+        else if (region == 3) x = a[k] + s * ab[k];
+        else if (region == 4) x = a[k] + t * ac[k];
+        else if (region == 5) x = b[k] + t * (cc[k] - b[k]);
+        else x = (a[k] + ab[k] * s) + ac[k] * t;
+        c[k] = x;
+        ok &= isfinite(x) != 0;
+    }
+    u = region == 1 ? 1.0f : (region == 3 || region == 6 ? s : (region == 5 ? 1.0f - t : 0.0f));
+    w = region == 2 ? 1.0f : (region >= 4 ? t : 0.0f);
+    ok &= isfinite(u) != 0 && isfinite(w) != 0;
+    if (!ok) {
+        float best = INFINITY;
+        int j = 0;
+#pragma unroll
+        for (int m = 0; m < 3; ++m) {
+            float e[3];
+#pragma unroll
+            for (int k = 0; k < 3; ++k) e[k] = v[3 * m + k] - p[k];
+            const float dd = mr_dot(e, e);
+            if (m == 0 || dd < best) { best = dd; j = m; }
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k) c[k] = v[3 * j + k];
+        u = j == 1 ? 1.0f : 0.0f;
+        w = j == 2 ? 1.0f : 0.0f;
+    }
+    float e[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) e[k] = c[k] - p[k];
+    return mr_dot(e, e);
+}
+
+// own box of a triangle, as mr_tri_hit takes it
+__host__ __device__ __forceinline__ void mr_tri_box(const float v[9], float lo[3], float hi[3]) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const float a = v[k], b = v[3 + k], c = v[6 + k];
+        lo[k] = a < b ? (a < c ? a : c) : (b < c ? b : c);
+        hi[k] = a > b ? (a > c ? a : c) : (b > c ? b : c);
+    }
+}
+
+__device__ __forceinline__ void mr_load_node(const MrNode *nodes, int node, float b[12], int &c0, int &c1) {
+    const float4 *q = reinterpret_cast<const float4 *>(nodes + node);
+    const float4 q0 = __ldg(q), q1 = __ldg(q + 1), q2 = __ldg(q + 2), q3 = __ldg(q + 3);
+    b[0] = q0.x; b[1] = q0.y; b[2] = q0.z; b[3] = q0.w; b[4] = q1.x; b[5] = q1.y;
+    b[6] = q1.z; b[7] = q1.w; b[8] = q2.x; b[9] = q2.y; b[10] = q2.z; b[11] = q2.w;
+    c0 = __float_as_int(q3.x);
+    c1 = __float_as_int(q3.y);
+}
+
+// closest triangle to p: d2 (its d^2, +inf with best < 0 when p is not finite or the scene is empty), the (g, p) key,
+// the leaf index, the point and its weights
+__device__ __forceinline__ void mr_closest(const char *__restrict__ bvh, const float p[3], float &d2b, unsigned long long &kb, int &best, float cb[3],
+                                           float &ub, float &wb) {
+    const int n_leaf = __ldg(reinterpret_cast<const int *>(bvh));
+    const MrNode *nodes = reinterpret_cast<const MrNode *>(bvh + mr_nodes_offset());
+    const MrTri *leaves = reinterpret_cast<const MrTri *>(bvh + mr_leaves_offset(n_leaf));
+    float keyb = INFINITY;
+    d2b = INFINITY; ub = 0.0f; wb = 0.0f;
+    cb[0] = cb[1] = cb[2] = 0.0f;
+    kb = ~0ull;
+    best = -1;
+    if (!(n_leaf > 0 && isfinite(p[0]) && isfinite(p[1]) && isfinite(p[2]))) return;
+    int stack[kMrStack];
+    int sp = 0;
+    int node = n_leaf > 1 ? 0 : ~0;
+    stack[sp++] = kMrEmpty;
+    while (node != kMrEmpty) {
+        while (node >= 0) {               // inner nodes: descend, nearest child (by lb) first
+            float b[12];
+            int c0, c1;
+            mr_load_node(nodes, node, b, c0, c1);
+            const float l0 = mr_box_lb(b, b + 3, p), l1 = mr_box_lb(b + 6, b + 9, p);
+            const bool h0 = !(l0 > keyb), h1 = !(l1 > keyb);
+            if (h0 && h1) {
+                const bool first0 = !(l1 < l0);
+                stack[sp++] = first0 ? c1 : c0;
+                node = first0 ? c0 : c1;
+            } else if (h0 || h1) {
+                node = h0 ? c0 : c1;
+            } else {
+                node = stack[--sp];
+            }
+        }
+        if (node != kMrEmpty) {           // a leaf
+            const int li = ~node;
+            float v[9], c[3], u, w, lo[3], hi[3];
+            uint32_t g, pr;
+            mr_load_tri(leaves, li, v, g, pr);
+            const float d2 = mr_closest_tri(p, v, c, u, w);
+            mr_tri_box(v, lo, hi);
+            const float lb = mr_box_lb(lo, hi, p);
+            const float key = d2 > lb ? d2 : lb;
+            const unsigned long long gp = (unsigned long long)g << 32 | pr;
+            if (key < keyb || (key == keyb && gp < kb)) {
+                keyb = key; kb = gp; best = li; d2b = d2; ub = u; wb = w;
+                cb[0] = c[0]; cb[1] = c[1]; cb[2] = c[2];
+            }
+            node = stack[--sp];
+        }
+    }
+}
+
+// accepted hits of the ray with tnear <= t <= tfar (ANY: stop at the first, return 0 or 1)
+template <bool ANY>
+__device__ __forceinline__ int mr_count(const char *__restrict__ bvh, const float r[6], float tnear, float tfar) {
+    const int n_leaf = __ldg(reinterpret_cast<const int *>(bvh));
+    const MrNode *nodes = reinterpret_cast<const MrNode *>(bvh + mr_nodes_offset());
+    const MrTri *leaves = reinterpret_cast<const MrTri *>(bvh + mr_leaves_offset(n_leaf));
+    MrRay ray;
+    if (!(n_leaf > 0 && mr_ray_setup(r, ray))) return 0;
+    int count = 0;
+    int stack[kMrStack];
+    int sp = 0;
+    int node = n_leaf > 1 ? 0 : ~0;
+    stack[sp++] = kMrEmpty;
+    while (node != kMrEmpty) {
+        while (node >= 0) {
+            float b[12], a0, b0, a1, b1;
+            int c0, c1;
+            mr_load_node(nodes, node, b, c0, c1);
+            mr_box_interval(b, b + 3, ray.o, ray.d, a0, b0);
+            mr_box_interval(b + 6, b + 9, ray.o, ray.d, a1, b1);
+            const bool h0 = !(a0 > tfar) && !(b0 < tnear) && !(a0 > b0), h1 = !(a1 > tfar) && !(b1 < tnear) && !(a1 > b1);
+            if (h0 && h1) {
+                const bool first0 = !(a1 < a0);
+                stack[sp++] = first0 ? c1 : c0;
+                node = first0 ? c0 : c1;
+            } else if (h0 || h1) {
+                node = h0 ? c0 : c1;
+            } else {
+                node = stack[--sp];
+            }
+        }
+        if (node != kMrEmpty) {
+            float v[9], t, u, w2;
+            uint32_t g, p;
+            mr_load_tri(leaves, ~node, v, g, p);
+            if (mr_tri_hit(ray, v, t, u, w2) && tnear <= t && t <= tfar) {
+                ++count;
+                if (ANY) return 1;
+            }
+            node = stack[--sp];
+        }
+    }
+    return count;
+}
+
+__device__ __forceinline__ void mr_load_point(const float *__restrict__ pts, int64_t i, float p[3]) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) p[k] = __ldg(pts + 3 * i + k);
+}
+
+// FULL: closest point, ids, uvs and unit normal (compute_closest_points); otherwise the distance sqrtf(d^2) only
+template <bool FULL>
+__global__ void __launch_bounds__(256) mesh_closest_kernel(const char *__restrict__ bvh, const float *__restrict__ pts, int64_t n, float *__restrict__ dist,
+                                                           float *__restrict__ points, uint32_t *__restrict__ geom_ids, uint32_t *__restrict__ prim_ids,
+                                                           float *__restrict__ uvs, float *__restrict__ normals) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float p[3], d2, c[3], u, w;
+    unsigned long long kb;
+    int best;
+    mr_load_point(pts, i, p);
+    mr_closest(bvh, p, d2, kb, best, c, u, w);
+    if constexpr (!FULL) {
+        dist[i] = sqrtf(d2);
+    } else {
+#pragma unroll
+        for (int k = 0; k < 3; ++k) points[3 * i + k] = c[k];
+        geom_ids[i] = best >= 0 ? (uint32_t)(kb >> 32) : kMrInvalid;
+        prim_ids[i] = best >= 0 ? (uint32_t)kb : kMrInvalid;
+        uvs[2 * i] = u;
+        uvs[2 * i + 1] = w;
+        float nv[3] = {0.0f, 0.0f, 0.0f};
+        if (best >= 0) {
+            const int n_leaf = __ldg(reinterpret_cast<const int *>(bvh));
+            float v[9], nn;
+            uint32_t g, pr;
+            mr_load_tri(reinterpret_cast<const MrTri *>(bvh + mr_leaves_offset(n_leaf)), best, v, g, pr);
+            mr_normal(v, nv, nn);
+            const float len = sqrtf(nn);
+#pragma unroll
+            for (int k = 0; k < 3; ++k) nv[k] = nv[k] / len;
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k) normals[3 * i + k] = nv[k];
+    }
+}
+
+// count_intersections (ANY = false, tnear = 0, tfar = +inf: int32 counts) and test_occlusions (ANY: uint8 0 / 1)
+template <bool ANY>
+__global__ void __launch_bounds__(256) mesh_count_kernel(const char *__restrict__ bvh, const float *__restrict__ rays, int64_t n, float tnear, float tfar,
+                                                         int32_t *__restrict__ counts, uint8_t *__restrict__ occluded) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float r[6];
+#pragma unroll
+    for (int k = 0; k < 6; ++k) r[k] = __ldg(rays + 6 * i + k);
+    const int c = mr_count<ANY>(bvh, r, tnear, tfar);
+    if (ANY) occluded[i] = (uint8_t)c;
+    else counts[i] = c;
+}
+
+// occupancy: 1 when more than half of the first dirs.n directions from p cross the surface an odd number of times.
+// SIGNED: sdist holds the distances (mesh_closest_kernel<false>, launched before on the same stream) and is negated
+// where the occupancy is 1 (compute_signed_distance).  Composing the two kernels measured faster than running the
+// closest-point traversal in this thread (DESIGN section 4).
+template <bool SIGNED>
+__global__ void __launch_bounds__(256) mesh_occupancy_kernel(const char *__restrict__ bvh, const float *__restrict__ pts, int64_t n, const __grid_constant__ MrDirs dirs,
+                                                             float *__restrict__ occupancy, float *__restrict__ sdist) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    float p[3];
+    mr_load_point(pts, i, p);
+    int inside = 0;
+    for (int s = 0; s < dirs.n; ++s) {
+        const float r[6] = {p[0], p[1], p[2], dirs.d[s][0], dirs.d[s][1], dirs.d[s][2]};
+        inside += mr_count<false>(bvh, r, 0.0f, INFINITY) & 1;
+    }
+    const bool occ = 2 * inside > dirs.n;
+    if (occupancy) occupancy[i] = occ ? 1.0f : 0.0f;
+    if (SIGNED && occ) sdist[i] = -sdist[i];
+}
+
+static unsigned mr_blocks(int64_t n) { return (unsigned)((n + 255) / 256); }
+
 // ------------------------------------------------------------------ build
 
 struct MrStatus {
@@ -631,6 +935,82 @@ int bslam_mesh_cast_pinhole(const void *d_bvh, int F, int H, int W, const double
         else mr_launch_pinhole<false, false>(grid, bvh, ph, t, g, p, uv, nrm, st);
         BSLAM_LAUNCH_CHECK();
     }
+    return BSLAM_OK;
+}
+
+int bslam_mesh_occupancy_directions(int n, float *h_dirs) {
+    BSLAM_CHECK_ARG(n >= 0 && n <= BSLAM_MESH_MAX_SAMPLES, "bslam_mesh_occupancy_directions: n = %d outside [0, %d]", n, BSLAM_MESH_MAX_SAMPLES);
+    BSLAM_CHECK_ARG(h_dirs || n == 0, "bslam_mesh_occupancy_directions: NULL argument");
+    bslam_mesh_direction_set(n, h_dirs);
+    return BSLAM_OK;
+}
+
+int bslam_mesh_closest_points(const void *d_bvh, const float *d_points, int64_t n, float *d_closest, uint32_t *d_geom_ids, uint32_t *d_prim_ids,
+                              float *d_uvs, float *d_normals, bslam_stream_t stream) {
+    BSLAM_CHECK_ARG(n >= 0, "bslam_mesh_closest_points: n = %lld < 0", (long long)n);
+    if (n == 0) return BSLAM_OK;
+    BSLAM_CHECK_ARG(d_bvh && d_points && d_closest && d_geom_ids && d_prim_ids && d_uvs && d_normals, "bslam_mesh_closest_points: NULL argument");
+    BSLAM_CHECK_ARG(n <= (int64_t)INT_MAX * 256, "bslam_mesh_closest_points: too many points (%lld)", (long long)n);
+    mesh_closest_kernel<true><<<mr_blocks(n), 256, 0, (cudaStream_t)stream>>>((const char *)d_bvh, d_points, n, nullptr, d_closest, d_geom_ids, d_prim_ids,
+                                                                               d_uvs, d_normals);
+    BSLAM_LAUNCH_CHECK();
+    return BSLAM_OK;
+}
+
+int bslam_mesh_distance(const void *d_bvh, const float *d_points, int64_t n, float *d_distance, bslam_stream_t stream) {
+    BSLAM_CHECK_ARG(n >= 0, "bslam_mesh_distance: n = %lld < 0", (long long)n);
+    if (n == 0) return BSLAM_OK;
+    BSLAM_CHECK_ARG(d_bvh && d_points && d_distance, "bslam_mesh_distance: NULL argument");
+    BSLAM_CHECK_ARG(n <= (int64_t)INT_MAX * 256, "bslam_mesh_distance: too many points (%lld)", (long long)n);
+    mesh_closest_kernel<false><<<mr_blocks(n), 256, 0, (cudaStream_t)stream>>>((const char *)d_bvh, d_points, n, d_distance, nullptr, nullptr, nullptr,
+                                                                                nullptr, nullptr);
+    BSLAM_LAUNCH_CHECK();
+    return BSLAM_OK;
+}
+
+int bslam_mesh_occupancy(const void *d_bvh, const float *d_points, int64_t n, int nsamples, float *d_occupancy, float *d_signed_distance,
+                         bslam_stream_t stream) {
+    BSLAM_CHECK_ARG(n >= 0, "bslam_mesh_occupancy: n = %lld < 0", (long long)n);
+    BSLAM_CHECK_ARG(nsamples >= 1 && nsamples <= BSLAM_MESH_MAX_SAMPLES && nsamples % 2 == 1,
+                    "bslam_mesh_occupancy: nsamples = %d must be odd and in [1, %d]", nsamples, BSLAM_MESH_MAX_SAMPLES);
+    if (n == 0) return BSLAM_OK;
+    BSLAM_CHECK_ARG(d_bvh && d_points && (d_occupancy || d_signed_distance), "bslam_mesh_occupancy: NULL argument");
+    BSLAM_CHECK_ARG(n <= (int64_t)INT_MAX * 256, "bslam_mesh_occupancy: too many points (%lld)", (long long)n);
+    MrDirs dirs;
+    dirs.n = nsamples;
+    bslam_mesh_direction_set(nsamples, &dirs.d[0][0]);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d_signed_distance) {
+        mesh_closest_kernel<false><<<mr_blocks(n), 256, 0, st>>>((const char *)d_bvh, d_points, n, d_signed_distance, nullptr, nullptr, nullptr, nullptr,
+                                                                 nullptr);
+        BSLAM_LAUNCH_CHECK();
+        mesh_occupancy_kernel<true><<<mr_blocks(n), 256, 0, st>>>((const char *)d_bvh, d_points, n, dirs, d_occupancy, d_signed_distance);
+    } else {
+        mesh_occupancy_kernel<false><<<mr_blocks(n), 256, 0, st>>>((const char *)d_bvh, d_points, n, dirs, d_occupancy, nullptr);
+    }
+    BSLAM_LAUNCH_CHECK();
+    return BSLAM_OK;
+}
+
+int bslam_mesh_count_intersections(const void *d_bvh, const float *d_rays, int64_t n, int32_t *d_counts, bslam_stream_t stream) {
+    BSLAM_CHECK_ARG(n >= 0, "bslam_mesh_count_intersections: n = %lld < 0", (long long)n);
+    if (n == 0) return BSLAM_OK;
+    BSLAM_CHECK_ARG(d_bvh && d_rays && d_counts, "bslam_mesh_count_intersections: NULL argument");
+    BSLAM_CHECK_ARG(n <= (int64_t)INT_MAX * 256, "bslam_mesh_count_intersections: too many rays (%lld)", (long long)n);
+    mesh_count_kernel<false><<<mr_blocks(n), 256, 0, (cudaStream_t)stream>>>((const char *)d_bvh, d_rays, n, 0.0f, INFINITY, d_counts, nullptr);
+    BSLAM_LAUNCH_CHECK();
+    return BSLAM_OK;
+}
+
+int bslam_mesh_test_occlusions(const void *d_bvh, const float *d_rays, int64_t n, float tnear, float tfar, uint8_t *d_occluded, bslam_stream_t stream) {
+    BSLAM_CHECK_ARG(n >= 0, "bslam_mesh_test_occlusions: n = %lld < 0", (long long)n);
+    BSLAM_CHECK_ARG(tnear >= 0.0f && !isnan(tfar), "bslam_mesh_test_occlusions: bad bounds (tnear=%g tfar=%g; tnear must be >= 0, neither NaN)",
+                    (double)tnear, (double)tfar);
+    if (n == 0) return BSLAM_OK;
+    BSLAM_CHECK_ARG(d_bvh && d_rays && d_occluded, "bslam_mesh_test_occlusions: NULL argument");
+    BSLAM_CHECK_ARG(n <= (int64_t)INT_MAX * 256, "bslam_mesh_test_occlusions: too many rays (%lld)", (long long)n);
+    mesh_count_kernel<true><<<mr_blocks(n), 256, 0, (cudaStream_t)stream>>>((const char *)d_bvh, d_rays, n, tnear, tfar, nullptr, d_occluded);
+    BSLAM_LAUNCH_CHECK();
     return BSLAM_OK;
 }
 

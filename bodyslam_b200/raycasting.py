@@ -7,6 +7,8 @@ section 7).  There is no CPU path.
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 
 from . import _lib, ops
@@ -15,6 +17,7 @@ from .geometry import to_numpy
 INVALID_ID = 0xFFFFFFFF
 _INDEX_DTYPES = ("int32", "int64", "uint32")
 _KEYS = ("t_hit", "geometry_ids", "primitive_ids", "primitive_uvs", "primitive_normals")   # C ABI output order
+MAX_OCCUPANCY_SAMPLES = 31          # BSLAM_MESH_MAX_SAMPLES: the size of the occupancy direction set
 
 
 def _mesh_arrays(mesh):
@@ -150,4 +153,88 @@ class RaycastingScene:
         with torch.cuda.device(self.device):
             _lib.check(L.bslam_mesh_cast_pinhole(_lib.ptr(bvh), F, H, W, _lib.ptr(K), _lib.ptr(E), *(_lib.ptr(out.get(k)) for k in _KEYS),
                                                  _lib.stream_ptr(self.device)))
+        return out
+
+    # ------------------------------------------------------------------ point and ray queries
+    # Semantics (tests/mesh_query_ref.c): the nearest triangle is the lexicographic minimum of (max(d^2, lb of its box),
+    # geometry, primitive) with Ericson's closest point; a query point with a non-finite component, or an empty scene,
+    # gives distance +inf, INVALID_ID and zeros.  `nthreads` is accepted for Open3D's positional order and ignored.
+
+    def _queries(self, x, width, what):
+        if ops._dtype_name(x) != "float32" or len(x.shape) < 1 or x.shape[-1] != width:
+            raise RuntimeError(f"RaycastingScene.{what}: expected float32 [..., {width}] (got {ops._dtype_name(x)} {tuple(x.shape)})")
+        q = ops.as_cuda(x, self.torch.float32, self.device)
+        return q, tuple(q.shape[:-1]), q.numel() // width
+
+    def compute_closest_points(self, query_points, nthreads: int = 0) -> dict:
+        """query_points [..., 3] float32 -> dict of CUDA tensors with the points' leading shape: points [..., 3] (the
+        closest point on the nearest triangle), geometry_ids / primitive_ids uint32, primitive_uvs [..., 2] (weights of
+        v1, v2) and primitive_normals [..., 3] (the cast's unit normal)."""
+        torch, L = self.torch, _lib.load()
+        q, lead, n = self._queries(query_points, 3, "compute_closest_points")
+        bvh = self._commit()
+        dev = self.device
+        out = {"points": torch.empty(lead + (3,), dtype=torch.float32, device=dev),
+               "geometry_ids": torch.empty(lead, dtype=torch.uint32, device=dev),
+               "primitive_ids": torch.empty(lead, dtype=torch.uint32, device=dev),
+               "primitive_uvs": torch.empty(lead + (2,), dtype=torch.float32, device=dev),
+               "primitive_normals": torch.empty(lead + (3,), dtype=torch.float32, device=dev)}
+        with torch.cuda.device(dev):
+            _lib.check(L.bslam_mesh_closest_points(_lib.ptr(bvh), _lib.ptr(q), n, *(_lib.ptr(x) for x in out.values()), _lib.stream_ptr(dev)))
+        return out
+
+    def compute_distance(self, query_points, nthreads: int = 0):
+        """query_points [..., 3] float32 -> float32 CUDA tensor [...]: distance to the nearest triangle"""
+        torch, L = self.torch, _lib.load()
+        q, lead, n = self._queries(query_points, 3, "compute_distance")
+        bvh = self._commit()
+        out = torch.empty(lead, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(L.bslam_mesh_distance(_lib.ptr(bvh), _lib.ptr(q), n, _lib.ptr(out), _lib.stream_ptr(self.device)))
+        return out
+
+    def _occupancy(self, query_points, nsamples, signed, what):
+        torch, L = self.torch, _lib.load()
+        q, lead, n = self._queries(query_points, 3, what)
+        ns = int(nsamples)
+        if ns != nsamples or ns < 1 or ns > MAX_OCCUPANCY_SAMPLES or ns % 2 == 0:
+            raise RuntimeError(f"RaycastingScene.{what}: nsamples must be odd and in [1, {MAX_OCCUPANCY_SAMPLES}] (got {nsamples})")
+        bvh = self._commit()
+        out = torch.empty(lead, dtype=torch.float32, device=self.device)
+        occ, sd = (None, out) if signed else (out, None)
+        with torch.cuda.device(self.device):
+            _lib.check(L.bslam_mesh_occupancy(_lib.ptr(bvh), _lib.ptr(q), n, ns, _lib.ptr(occ), _lib.ptr(sd), _lib.stream_ptr(self.device)))
+        return out
+
+    def compute_signed_distance(self, query_points, nthreads: int = 0, nsamples: int = 1):
+        """query_points [..., 3] float32 -> float32 CUDA tensor [...]: the distance, negative where compute_occupancy
+        is 1"""
+        return self._occupancy(query_points, nsamples, True, "compute_signed_distance")
+
+    def compute_occupancy(self, query_points, nthreads: int = 0, nsamples: int = 1):
+        """query_points [..., 3] float32 -> float32 CUDA tensor [...] of 0 / 1: 1 when more than half of nsamples rays
+        (odd, <= 31, along a fixed direction set) from the point cross the meshes an odd number of times"""
+        return self._occupancy(query_points, nsamples, False, "compute_occupancy")
+
+    def count_intersections(self, rays, nthreads: int = 0):
+        """rays [..., 6] float32 -> int32 CUDA tensor [...]: the number of triangles the cast accepts at any t >= 0 (a
+        ray through an edge shared by two triangles counts both)"""
+        torch, L = self.torch, _lib.load()
+        r, lead, n = self._queries(rays, 6, "count_intersections")
+        bvh = self._commit()
+        out = torch.empty(lead, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(L.bslam_mesh_count_intersections(_lib.ptr(bvh), _lib.ptr(r), n, _lib.ptr(out), _lib.stream_ptr(self.device)))
+        return out
+
+    def test_occlusions(self, rays, tnear: float = 0.0, tfar: float = math.inf, nthreads: int = 0):
+        """rays [..., 6] float32 -> bool CUDA tensor [...]: some accepted hit with tnear <= t <= tfar (both inclusive;
+        tnear >= 0, neither bound NaN; the bounds are rounded to float32)"""
+        torch, L = self.torch, _lib.load()
+        r, lead, n = self._queries(rays, 6, "test_occlusions")
+        bvh = self._commit()
+        out = torch.empty(lead, dtype=torch.bool, device=self.device)
+        with torch.cuda.device(self.device):
+            _lib.check(L.bslam_mesh_test_occlusions(_lib.ptr(bvh), _lib.ptr(r), n, float(np.float32(tnear)), float(np.float32(tfar)), _lib.ptr(out),
+                                                    _lib.stream_ptr(self.device)))
         return out

@@ -498,6 +498,33 @@ BSLAM_API int bslam_mesh_rays_pinhole(int F, int H, int W, const double *h_K, co
 BSLAM_API int bslam_mesh_cast_pinhole(const void *d_bvh, int F, int H, int W, const double *h_K, const double *h_extrinsics, float *d_t_hit,
                                       uint32_t *d_geom_ids, uint32_t *d_prim_ids, float *d_uvs, float *d_normals, bslam_stream_t stream);
 
+/* Point and ray queries of the same BVH (Open3D's compute_closest_points, compute_distance, compute_occupancy,
+ * compute_signed_distance, count_intersections, test_occlusions), equal bit for bit to tests/mesh_query_ref.c; one
+ * thread per query, no synchronisation.  n == 0 launches nothing and accepts NULL buffers.
+ *
+ * bslam_mesh_closest_points: d_points [n][3] f32 -> d_closest [n][3] (Ericson's closest point on the nearest triangle),
+ * geometry / primitive ids, d_uvs [n][2] (weights of v1, v2) and d_normals [n][3] (unit, as the cast's), all required.
+ * Nearest = lexicographic minimum of (max(d^2, lb(triangle box)), g, p).  A point with a non-finite component, or an
+ * empty scene: ids 0xFFFFFFFF, everything else 0.  bslam_mesh_distance: d_distance [n] = sqrtf(d^2) of that triangle
+ * (+inf for such points).
+ * bslam_mesh_occupancy: rays from each point along the first nsamples directions of bslam_mesh_occupancy_directions;
+ * occupancy 1.0f when more than half of them have an odd intersection count, else 0.0f (0 for non-finite points).
+ * nsamples must be odd and at most BSLAM_MESH_MAX_SAMPLES (31).  d_occupancy and d_signed_distance are optional (one is
+ * required): the signed distance is the distance, negated when the occupancy is 1.
+ * bslam_mesh_count_intersections: d_counts [n] i32 = number of triangles the cast would accept for the ray at any
+ * t >= 0 (a ray through a shared edge counts both triangles).  bslam_mesh_test_occlusions: d_occluded [n] u8 = 1 iff
+ * some accepted hit has tnear <= t <= tfar (inclusive); tnear < 0 or a NaN bound is an argument error.
+ * bslam_mesh_occupancy_directions: the float32 directions [n][3] (host), n <= 31. */
+BSLAM_API int bslam_mesh_closest_points(const void *d_bvh, const float *d_points, int64_t n, float *d_closest, uint32_t *d_geom_ids, uint32_t *d_prim_ids,
+                                        float *d_uvs, float *d_normals, bslam_stream_t stream);
+BSLAM_API int bslam_mesh_distance(const void *d_bvh, const float *d_points, int64_t n, float *d_distance, bslam_stream_t stream);
+BSLAM_API int bslam_mesh_occupancy(const void *d_bvh, const float *d_points, int64_t n, int nsamples, float *d_occupancy, float *d_signed_distance,
+                                   bslam_stream_t stream);
+BSLAM_API int bslam_mesh_count_intersections(const void *d_bvh, const float *d_rays, int64_t n, int32_t *d_counts, bslam_stream_t stream);
+BSLAM_API int bslam_mesh_test_occlusions(const void *d_bvh, const float *d_rays, int64_t n, float tnear, float tfar, uint8_t *d_occluded,
+                                         bslam_stream_t stream);
+BSLAM_API int bslam_mesh_occupancy_directions(int n, float *h_dirs);
+
 /* Surface-extraction flavour of bslam_mc_* / bslam_points_*: a voxel is valid when weight >= weight_threshold
  * (0 = weight > 0, Open3D's legacy `weight != 0` for every weight an integrator writes: they differ only for negative
  * or NaN weights, which count as invalid here; the tensor pipeline's extract_triangle_mesh / extract_point_cloud default

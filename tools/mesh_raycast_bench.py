@@ -52,11 +52,8 @@ def events_ms(fn, n):
     return a.elapsed_time(b) / n
 
 
-def main():
-    if not torch.cuda.is_available():
-        raise SystemExit("mesh_raycast_bench: needs a CUDA device")
-    dev = torch.device("cuda", 0)
-    out = {"metric": "mesh_raycast", "gpu": gpu_info()}
+def reconstruction(dev):
+    """configs[3] integrated in full and its marching-cubes mesh -> (mesh, cfg, extrinsics, intrinsic)"""
     cfg = S.config("laparoscopy512")
     F, W, H, K = cfg["frames"], cfg["W"], cfg["H"], cfg["K"]
     E = cfg["extrinsics"](F)
@@ -69,6 +66,16 @@ def main():
     del depth_u16
     mesh = vol.extract_triangle_mesh()
     del vol
+    return mesh, cfg, E, intr
+
+
+def main():
+    if not torch.cuda.is_available():
+        raise SystemExit("mesh_raycast_bench: needs a CUDA device")
+    dev = torch.device("cuda", 0)
+    out = {"metric": "mesh_raycast", "gpu": gpu_info()}
+    mesh, cfg, E, intr = reconstruction(dev)
+    F, W, H = cfg["frames"], cfg["W"], cfg["H"]
     n_tris = int(mesh.triangles.shape[0])
     out["mesh"] = {"source": f"laparoscopy512 {cfg['resolution']}^3, {F} frames, extract_triangle_mesh", "triangles": n_tris,
                    "vertices": int(mesh.vertices.shape[0])}
