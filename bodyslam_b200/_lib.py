@@ -29,7 +29,7 @@ _SIGNATURES = {
     "bslam_colorize_f32": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, _p, _p, C.c_double, C.c_double, C.c_int, C.c_float, C.c_uint32, _p, _p, _p, _p]),
     "bslam_minmax_u8": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p, _p]),
     "bslam_median_u16": (C.c_int, [_p, C.c_int, C.c_int64, C.c_int, C.c_uint16, _p, _p, _p]),
-    "bslam_depth_from_u16": (C.c_int, [_p, C.c_int64, C.c_float, C.c_float, _p, _p]),
+    "bslam_depth_from_u16": (C.c_int, [_p, C.c_int64, C.c_float, C.c_double, _p, _p]),
     "bslam_backproject_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "bslam_backproject": (C.c_int, [_p, _p, C.c_int, C.c_int, C.c_int, C.c_int, _p, _p, C.c_int, _p, _p, C.c_int64, _p, _p, _p]),
     "bslam_tsdf_storage_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
@@ -38,11 +38,11 @@ _SIGNATURES = {
     "bslam_tsdf_destroy": (C.c_int, [_p]),
     "bslam_tsdf_reset": (C.c_int, [_p, _p]),
     "bslam_tsdf_copy": (C.c_int, [_p, _p, _p]),
-    "bslam_tsdf_unit_bounds": (C.c_int, [_p, _p, C.c_int, C.c_float, C.c_float, C.c_int, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p, _p]),
+    "bslam_tsdf_unit_bounds": (C.c_int, [_p, _p, C.c_int, C.c_float, C.c_double, C.c_int, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p, _p]),
     "bslam_tsdf_grow_box": (C.c_int, [_p, _p, _p, _p, _p, _p]),
     "bslam_tsdf_integrate": (C.c_int, [_p, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, C.c_int, _p, C.c_int, _p]),
-    "bslam_tsdf_integrate_u16": (C.c_int, [_p, _p, C.c_float, C.c_float, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p]),
-    "bslam_tsdf_prepare_u16": (C.c_int, [_p, _p, C.c_float, C.c_float, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p]),
+    "bslam_tsdf_integrate_u16": (C.c_int, [_p, _p, C.c_float, C.c_double, _p, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p, _p]),
+    "bslam_tsdf_prepare_u16": (C.c_int, [_p, _p, C.c_float, C.c_double, _p, C.c_int, C.c_int, C.c_int, _p, _p, _p]),
     "bslam_tsdf_integrate_prepared": (C.c_int, [_p, _p, _p, _p]),
     "bslam_tsdf_set_z_interleave": (C.c_int, [_p, C.c_int]),
     "bslam_tsdf_layout": (C.c_int, [_p, _p]),

@@ -7,7 +7,10 @@
 //   q      = float32(p) / float32(100);  virt = float32(n - 1) * q            (float32 products)
 //   i0     = floor(virt), i1 = min(i0 + 1, n - 1), gamma = virt - i0           (float32)
 //   vmin   = lerp(sorted[i0], sorted[i1], gamma)  with numpy's _lerp           (float32)
+//            NaN when any valid pixel is NaN (np.percentile propagates NaN), so every valid pixel gets the bad colour
 //   x      = (value - vmin) / (vmax - vmin)   (float32)   or   value * 0  when vmin == vmax
+//            with both bounds explicit (Python floats) `vmin != vmax` and `vmax - vmin` are evaluated in double,
+//            and the difference meets the float32 array rounded to float32 (NEP 50)
 //   index  = matplotlib Colormap.__call__(x, bytes=True): x * 256, < 0 -> 0, == 256 -> 255, > 255 -> 255, trunc
 // The four order statistics come from an exact two-level radix select on the order-preserving 32-bit key of
 // the float: a 65 536-bin histogram of the key's high half, then -- for the (at most four) bins that hold a
@@ -22,11 +25,14 @@ constexpr int kFBins = 65536;
 // per-image workspace: hi histogram | 4 lo histograms | select state
 struct FSel {
     unsigned int n_valid;
+    unsigned int n_nan;         // valid pixels that are NaN (counted by the level-0 histogram pass)
     unsigned int want[4];       // wanted sorted positions
     unsigned int hi_bin[4];     // high half of the key holding each wanted position
     unsigned int before[4];     // valid pixels with a smaller high half
     float gamma[2];
     float vmin, vmax;
+    float den;                  // vmax - vmin as the normalisation divides by it
+    unsigned int flat;          // vmin == vmax: x = value * 0
 };
 constexpr size_t kFWsPerImage = (size_t)kFBins * 4 * 5 + 256;
 
@@ -56,11 +62,11 @@ __global__ void __launch_bounds__(256) fkey_hist_kernel(const float *__restrict_
     const int b = blockIdx.y;
     const float *img = value + (int64_t)b * n_per_image;
     unsigned int *hi = f_hist_hi(ws, b);
+    FSel *sel = f_sel(ws, b);
     unsigned int tgt[4] = {0, 0, 0, 0};
     if (LEVEL == 1) {
-        const FSel *s = f_sel(ws, b);
 #pragma unroll
-        for (int j = 0; j < 4; ++j) tgt[j] = s->hi_bin[j];
+        for (int j = 0; j < 4; ++j) tgt[j] = sel->hi_bin[j];
     }
     const int64_t per_iter = (int64_t)gridDim.x * blockDim.x;
     const int64_t n_round = (n_per_image + per_iter - 1) / per_iter * per_iter;   // whole warps stay converged for the ballots
@@ -74,6 +80,8 @@ __global__ void __launch_bounds__(256) fkey_hist_kernel(const float *__restrict_
         const unsigned int k = fkey(v);
         if (LEVEL == 0) {
             warp_hist_add(hi, k >> 16, ok);
+            const unsigned int nan = __ballot_sync(0xffffffffu, ok && v != v);
+            if (nan && (threadIdx.x & 31) == 0) atomicAdd(&sel->n_nan, (unsigned int)__popc(nan));
         } else {
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
@@ -202,13 +210,18 @@ __global__ void __launch_bounds__(1024) fkey_select_lo_kernel(void *ws, const do
         if (n > 0) {
             vmin = numpy_lerp_f32(s_val[0], s_val[1], s->gamma[0]);
             vmax = numpy_lerp_f32(s_val[2], s_val[3], s->gamma[1]);
+            if (s->n_nan) vmin = vmax = __int_as_float(0x7fffffff);   // np.percentile of data holding a NaN
         }
-        if (vmin_vmax_override) {           // explicit vmin / vmax: a Python float meets a float32 array -> float32 (NEP 50)
-            const double a = vmin_vmax_override[2 * b], c = vmin_vmax_override[2 * b + 1];
-            if (a == a) vmin = (float)a;
-            if (c == c) vmax = (float)c;
+        const double a = vmin_vmax_override ? vmin_vmax_override[2 * b] : NAN, c = vmin_vmax_override ? vmin_vmax_override[2 * b + 1] : NAN;
+        if (a == a) vmin = (float)a;        // explicit vmin / vmax: a Python float meets a float32 array -> float32 (NEP 50)
+        if (c == c) vmax = (float)c;
+        bool flat = vmin == vmax;
+        float den = vmax - vmin;
+        if (a == a && c == c) {             // two Python floats: compared and subtracted in double
+            flat = a == c;
+            den = (float)(c - a);
         }
-        s->vmin = vmin; s->vmax = vmax;
+        s->vmin = vmin; s->vmax = vmax; s->den = den; s->flat = flat;
         if (vmin_vmax_out) { vmin_vmax_out[2 * b] = (double)vmin; vmin_vmax_out[2 * b + 1] = (double)vmax; }
     }
 }
@@ -220,9 +233,8 @@ __global__ void __launch_bounds__(256) apply_f32_kernel(const float *__restrict_
     s_lut[threadIdx.x] = reinterpret_cast<const uint32_t *>(lut)[threadIdx.x];
     __syncthreads();
     const FSel *s = f_sel(ws, b);
-    const float vmin = s->vmin, vmax = s->vmax;
-    const bool flat = vmin == vmax;
-    const float den = vmax - vmin;
+    const float vmin = s->vmin, den = s->den;
+    const bool flat = s->flat != 0;
     const int64_t img_off = (int64_t)b * n_per_image;
     uint32_t *o32 = reinterpret_cast<uint32_t *>(out) + img_off;
     for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n_per_image; p += (int64_t)gridDim.x * blockDim.x) {

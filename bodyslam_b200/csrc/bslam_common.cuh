@@ -1,6 +1,7 @@
 // Shared host/device helpers of libbodyslam_b200 (sm_100a only).
 #pragma once
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
@@ -39,6 +40,19 @@ constexpr int kNumSMsB200 = 148;                    // B200 (compile-time sizing
 // same value); grids of the persistent kernels are sized from it, not from a constant.
 int num_sms(int device);
 int current_device_sms();
+
+// The depth truncation of the a4 conversion, as the f32 threshold the kernels compare against.  Open3D tests
+// `p >= depth_trunc` with p float32 and depth_trunc a double; for the smallest float t_f >= depth_trunc,
+// `p >= t_f` holds exactly when `(double)p >= depth_trunc` (a float p >= depth_trunc is >= t_f by minimality,
+// and p >= t_f >= depth_trunc the other way).  Rounding to nearest instead would drop the depths that lie
+// between depth_trunc and a t_f rounded below it (u = 3300 at scale 1000, trunc 3.3).  depth_trunc <= 0 or
+// NaN -> 0, which the kernels read as "no truncation"; +inf (or beyond FLT_MAX) -> +inf, which no depth reaches.
+inline float a4_trunc_threshold(double depth_trunc) {
+    if (!(depth_trunc > 0.0)) return 0.0f;
+    float t = (float)depth_trunc;
+    if ((double)t < depth_trunc) t = nextafterf(t, INFINITY);
+    return t;
+}
 
 // Every entry point that touches a volume runs on the volume's device and restores the caller's
 // current device on the way out (torch reads it through cudaGetDevice).

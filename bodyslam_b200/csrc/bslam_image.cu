@@ -754,11 +754,11 @@ int bslam_median_u16(const uint16_t *d_u16, int B, int64_t n_per_image, int has_
     return BSLAM_OK;
 }
 
-int bslam_depth_from_u16(const uint16_t *d_in, int64_t n, float depth_scale, float depth_trunc, float *d_out, bslam_stream_t stream) {
+int bslam_depth_from_u16(const uint16_t *d_in, int64_t n, float depth_scale, double depth_trunc, float *d_out, bslam_stream_t stream) {
     BSLAM_CHECK_ARG(d_in && d_out && n >= 0 && depth_scale > 0, "bslam_depth_from_u16: bad argument");
     BSLAM_CHECK_ARG(((uintptr_t)d_in & 7) == 0 && ((uintptr_t)d_out & 15) == 0, "bslam_depth_from_u16: buffers must be 16-byte aligned");
     if (n == 0) return BSLAM_OK;
-    depth_from_u16_kernel<<<grid_for(n, 1024), 256, 0, (cudaStream_t)stream>>>(d_in, n, depth_scale, depth_trunc, d_out);
+    depth_from_u16_kernel<<<grid_for(n, 1024), 256, 0, (cudaStream_t)stream>>>(d_in, n, depth_scale, a4_trunc_threshold(depth_trunc), d_out);
     BSLAM_LAUNCH_CHECK();
     return BSLAM_OK;
 }

@@ -95,7 +95,9 @@ BSLAM_API int bslam_colorize(const float *d_depth_m, const uint16_t *d_u16_in, i
  * both, depth_map_scaling.py:14-15): same steps as bslam_colorize, in NumPy's float32 arithmetic
  * (percentile virtual index, lerp, normalisation all float32, as NumPy 2.x evaluates them for a float32 array);
  * the order statistics come from an exact two-level radix select on the floats' order-preserving keys.
- * invalid_val is compared as float (`value == invalid_val`); NaN pixels get the colormap's "bad" colour (0,0,0,0).
+ * invalid_val is compared as float (`value == invalid_val`, so -0.0 matches +0.0 and NaN matches nothing).  Like
+ * np.percentile, a computed vmin / vmax is NaN when any valid pixel is NaN: every valid pixel of that image then gets
+ * the colormap's "bad" colour (0,0,0,0) (an explicit h_vmin_vmax side stays as given; the other side is still NaN).
  * d_workspace: bslam_colorize_f32_workspace_bytes(B).  h_vmin_vmax / d_vmin_vmax_out as in bslam_colorize.
  */
 BSLAM_API size_t bslam_colorize_f32_workspace_bytes(int B);
@@ -119,10 +121,13 @@ BSLAM_API int bslam_median_u16(const uint16_t *d_u16, int B, int64_t n_per_image
 
 /* ------------------------------------------------------------------ 3DM depth scaling (a4)
  * Replaces Open3D RGBDImage.create_from_color_and_depth(depth_scale, depth_trunc) as called at
- * N/3DM/slam_utils.py:212-220:  d = (float)u16 / (float)depth_scale;  d >= depth_trunc -> 0.
- * depth_trunc <= 0 disables truncation (the cv2 variant, slam_utils.py:231-233). */
+ * N/3DM/slam_utils.py:212-220:  d = (float)u16 / (float)depth_scale;  d >= depth_trunc -> 0, compared as
+ * Open3D does, (double)d >= depth_trunc (the kernels compare d against the smallest float >= depth_trunc, which
+ * is the same test).  The fused conversions of bslam_tsdf_integrate_u16 / bslam_tsdf_prepare_u16 /
+ * bslam_tsdf_unit_bounds apply the same rule.  depth_trunc <= 0 (or NaN) disables truncation (the cv2 variant,
+ * slam_utils.py:231-233); +inf truncates nothing. */
 BSLAM_API int bslam_depth_from_u16(const uint16_t *d_in, int64_t n, float depth_scale,
-                                   float depth_trunc, float *d_out, bslam_stream_t stream);
+                                   double depth_trunc, float *d_out, bslam_stream_t stream);
 
 /* Host helper: n row-major 4x4 float64 matrices inverted by the cofactor (adjugate / determinant) formula, the one
  * Eigen's Matrix4d::inverse() evaluates for Open3D's `extrinsic.inverse()` -- the camera pose of back-projection and
@@ -188,7 +193,7 @@ BSLAM_API int bslam_tsdf_copy(const bslam_volume *src, bslam_volume *dst, bslam_
 #define BSLAM_GROW_GROWN 1
 #define BSLAM_GROW_CAP_UNITS 2
 #define BSLAM_GROW_CAP_ROW_WORDS 3
-BSLAM_API int bslam_tsdf_unit_bounds(bslam_volume *vol, const void *d_depth, int depth_is_u16, float depth_scale, float depth_trunc,
+BSLAM_API int bslam_tsdf_unit_bounds(bslam_volume *vol, const void *d_depth, int depth_is_u16, float depth_scale, double depth_trunc,
                                      int F, int H, int W, int sampled, const double *h_K, const double *h_extrinsics,
                                      long long *h_bounds6, int *h_valid, bslam_stream_t stream);
 BSLAM_API int bslam_tsdf_grow_box(const long long *h_u0, const long long *h_nu, const long long *h_bounds6,
@@ -220,7 +225,7 @@ BSLAM_API int bslam_tsdf_integrate(bslam_volume *vol, const float *d_depth, cons
  * (what bslam_depth_from_u16 would have produced) and must stay valid until the call's work is done.
  */
 BSLAM_API int bslam_tsdf_integrate_u16(bslam_volume *vol, const uint16_t *d_depth_u16, float depth_scale,
-                                       float depth_trunc, float *d_depth_scratch, const uint8_t *d_rgb,
+                                       double depth_trunc, float *d_depth_scratch, const uint8_t *d_rgb,
                                        int F, int H, int W, const double *h_K, const double *h_extrinsics,
                                        unsigned long long *d_update_counts, bslam_stream_t stream);
 
@@ -233,7 +238,7 @@ BSLAM_API int bslam_tsdf_integrate_u16(bslam_volume *vol, const uint16_t *d_dept
  * preparation of chunk k+1 runs in the SM slots the tail of chunk k's integration leaves idle.  Frame order =
  * preparation order.  The buffers handed to prepare must stay valid until the matching integration is done.
  */
-BSLAM_API int bslam_tsdf_prepare_u16(bslam_volume *vol, const uint16_t *d_depth_u16, float depth_scale, float depth_trunc,
+BSLAM_API int bslam_tsdf_prepare_u16(bslam_volume *vol, const uint16_t *d_depth_u16, float depth_scale, double depth_trunc,
                                      float *d_depth_scratch, int F, int H, int W, const double *h_K, const double *h_extrinsics,
                                      bslam_stream_t prep_stream);
 BSLAM_API int bslam_tsdf_integrate_prepared(bslam_volume *vol, const uint8_t *d_rgb, unsigned long long *d_update_counts,

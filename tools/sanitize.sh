@@ -1,8 +1,8 @@
 #!/bin/bash
 # compute-sanitizer over the hot path (run on a GPU box):  bash tools/sanitize.sh > gpurun_out/sanitizer.log
 # memcheck + racecheck + synccheck on smoke() (a4, K3 with named barriers / shared flag words / persistent
-# claims, K4 marching cubes, K1, K2), on a small sharded-layout / unit-activation / colour integration and on colour
-# integrations whose RGB batches end exactly where their allocations do.
+# claims, K4 marching cubes, K1, K2), on a small sharded-layout / unit-activation / colour integration, on colour
+# integrations whose RGB batches end exactly where their allocations do, and on the image kernels at their edges.
 set -u
 CS=/usr/local/cuda/bin/compute-sanitizer
 PY='
@@ -28,6 +28,16 @@ for kw in (dict(unit_activation=True), dict(gz0=8, z_total=64, z_interleave=2), 
         if "gz0" not in kw:
             v.extract_triangle_mesh(); v.extract_point_cloud()
 mdem.colorize(np.random.default_rng(0).uniform(0.1, 3, (120, 160)).astype(np.float32), cmap="viridis", invalid_val=0)
+# image kernels at their edges: a K1 batch of 65 images of 45 x 101 px (H*W = 1 mod 4: every image after the first
+# off a 16-byte boundary), a K2 call of 130 frames (three emit chunks of poses) and a K1f image holding NaN pixels
+rng = np.random.default_rng(1)
+ops.colorize_u16(mdem.get_cmap_lut("viridis"), depth_u16=rng.integers(0, 65536, (65, 45, 101)).astype(np.uint16), invalid_val=0)
+bpd = rng.uniform(0.05, 3.0, (130, 30, 40)).astype(np.float32)
+bpd[rng.uniform(size=bpd.shape) < 0.1] = 0
+ops.backproject(bpd, (37.5, 36.0, 19.3, 15.1), np.eye(4)[None].repeat(130, 0), color=rng.integers(0, 256, (130, 30, 40, 3)).astype(np.uint8))
+fnan = rng.uniform(0.2, 4.0, (37, 23)).astype(np.float32)
+fnan.reshape(-1)[::7] = np.nan
+ops.colorize_f32(mdem.get_cmap_lut("viridis"), fnan, invalid_val=0.0)
 # colour gathers at the end of the RGB batch (PYTORCH_NO_CUDA_MEMORY_CACHING=1 below: every tensor is its own exactly sized
 # cudaMalloc): the 512 x 512 x 144 laparoscopy slab (8 z layers per warp, no long-chain phase), then 3 frames of 333 x 201
 # px, whose RGB batch (200 799 pixels) ends 3 bytes short of a 4-byte word
