@@ -299,3 +299,53 @@ def test_c_abi_argument_errors_do_not_need_a_device():
     assert track(P=65536) == _lib.E_ARG and b"65535" in L.bslam_last_error()
     assert L.bslam_odom_workspace_bytes(0, H, W, 2) == 0 and L.bslam_odom_workspace_bytes(3, 8, 8, 5) == 0
     assert L.bslam_odom_workspace_bytes(3, 480, 640, 3) >= 3 * 300 * 29 * 8
+
+
+# Huber parameter sets (depth_outlier_trunc, depth_huber_delta, intensity_huber_delta) and the branches each puts at
+# least 30 % of the inliers in, for the residual of each method: on the cavity pair below at the identity pose the
+# point-to-plane residuals stay under 0.05 and 90 % of the photometric ones under 0.1, so the defaults exercise the
+# quadratic branch only; (0.07, 0.002, 0.01) splits both residuals of the hybrid and the point-to-plane residual, and
+# sends 89 % of the intensity residuals to the linear branch; deltas of 0 put every non-zero residual in the linear
+# branch, 1e3 every residual in the quadratic one.
+HUBER_SETS = {(0.07, 0.05, 0.1): {R.POINT_TO_PLANE: {"depth": "q"}, R.INTENSITY: {"intensity": "q"}, R.HYBRID: {"intensity": "q", "depth": "q"}},
+              (0.07, 0.002, 0.01): {R.POINT_TO_PLANE: {"depth": "ql"}, R.INTENSITY: {"intensity": "l"}, R.HYBRID: {"intensity": "ql", "depth": "ql"}},
+              (0.07, 0.0, 0.0): {R.POINT_TO_PLANE: {"depth": "l"}, R.INTENSITY: {"intensity": "l"}, R.HYBRID: {"intensity": "l", "depth": "l"}},
+              (0.07, 1e3, 1e3): {R.POINT_TO_PLANE: {"depth": "q"}, R.INTENSITY: {"intensity": "q"}, R.HYBRID: {"intensity": "q", "depth": "q"}}}
+
+
+@pytest.fixture(scope="module")
+def cavity_pair():
+    E = S.cavity_sweep(1000)[:2]
+    d, c = S.render(S.Cavity(), E, K=S.K_640)
+    return R.Frames(d.numpy(), c.numpy(), S.K_640, 2), E[1] @ np.linalg.inv(E[0])
+
+
+@pytest.mark.parametrize("params", list(HUBER_SETS), ids=lambda p: "-".join(map(str, p)))
+@pytest.mark.parametrize("method", [R.POINT_TO_PLANE, R.INTENSITY, R.HYBRID])
+def test_linearize_matches_float64_restatement(cavity_pair, method, params):
+    """the mirror's 29 sums against odometry_ref.linearize_f64, an independent float64 evaluation of the same
+    linearisation.  Tolerance: linearize_f64's `tol`, derived there from the float32 rounding of J, r and the Huber terms
+    (running error analysis, <= 24 roundings of u = 2^-24 each relative to the operands' magnitudes) plus the whole terms
+    of the pixels whose projection or rejection decision lies within that bound of its threshold.  Measured over these
+    cases: the differences reach at most 4.5 % of the bound, the bound at most 0.35 % of the largest entry of AᵀA, and
+    at most 0.19 % of the inliers are ambiguous."""
+    fr, truth = cavity_pair
+    for level, T in ((0, np.eye(4)), (1, truth)):
+        ref = fr.linearize(0, 1, level, T, method, params)
+        f = R.linearize_f64(fr, 0, 1, level, T, method, params)
+        assert f["inliers"] > 50000 >> (2 * level), level
+        assert abs(ref[28] - f["sums"][28]) <= f["ambiguous"], (level, ref[28], f["sums"][28], f["ambiguous"])
+        assert np.all(np.abs(ref[:28] - f["sums"][:28]) <= f["tol"][:28]), (level, np.abs(ref - f["sums"]) / f["tol"])
+        # the bound stays far below a wrong branch's effect: 1 % of the largest entry of AᵀA (measured 0.35 %)
+        assert np.all(f["tol"][:21] <= 1e-2 * np.abs(f["sums"][:21]).max()), level
+        if level == 0:                    # the branch coverage this set claims (identity pose, as in HUBER_SETS)
+            n = f["inliers"]
+            for name, claim in HUBER_SETS[params][method].items():
+                quad, lin = f["branches"][name]
+                assert quad + lin == n
+                if "q" in claim:
+                    assert quad >= 0.3 * n, (name, quad, n)
+                if "l" in claim:
+                    assert lin >= 0.3 * n, (name, lin, n)
+            if params[1] == 0.0:          # all-linear with delta 0: no gradient, no loss
+                assert np.all(ref[21:28] == 0) and np.all(f["sums"][21:28] == 0)
