@@ -249,14 +249,23 @@ ORC_API int64_t orc_scalable_integrate(float *tsdf, float *weight, float *color,
                 const double z = (double)p;
                 const double x = (j - cxd) * z / fxd;
                 const double y = (i - cyd) * z / fyd;
+                double w[3];
+                int finite = 1;
+                for (int r = 0; r < 3; ++r) {
+                    w[r] = ((M[4 * r + 0] * x + M[4 * r + 1] * y) + M[4 * r + 2] * z) + M[4 * r + 3];
+                    finite &= isfinite(w[r]) != 0;
+                }
+                /* not finite: Open3D's (int) conversion gives the INT_MIN unit, outside every box */
+                if (!finite) continue;
+                const int n[3] = {nux, nuy, nuz};
                 int lo[3], hi[3];
                 for (int r = 0; r < 3; ++r) {
-                    const double w = ((M[4 * r + 0] * x + M[4 * r + 1] * y) + M[4 * r + 2] * z) + M[4 * r + 3];
-                    lo[r] = (int)floor((w - sdf_trunc) / unit_length) - unit0[r];
-                    hi[r] = (int)floor((w + sdf_trunc) / unit_length) - unit0[r];
+                    /* floor clamped to +-2^40 before the conversion, offset and clamp to the box in 64 bits: no UB for huge depths */
+                    const long long l = (long long)fmin(fmax(floor((w[r] - sdf_trunc) / unit_length), -1099511627776.0), 1099511627776.0) - unit0[r];
+                    const long long h = (long long)fmin(fmax(floor((w[r] + sdf_trunc) / unit_length), -1099511627776.0), 1099511627776.0) - unit0[r];
+                    lo[r] = (int)(l < 0 ? 0 : (l > n[r] ? n[r] : l));
+                    hi[r] = (int)(h > n[r] - 1 ? n[r] - 1 : (h < -1 ? -1 : h));
                 }
-                const int n[3] = {nux, nuy, nuz};
-                for (int r = 0; r < 3; ++r) { if (lo[r] < 0) lo[r] = 0; if (hi[r] > n[r] - 1) hi[r] = n[r] - 1; }
                 for (int ux = lo[0]; ux <= hi[0]; ++ux)
                     for (int uy = lo[1]; uy <= hi[1]; ++uy)
                         for (int uz = lo[2]; uz <= hi[2]; ++uz) touched[((size_t)ux * nuy + uy) * nuz + uz] = 1;

@@ -170,6 +170,64 @@ def test_scalable_units_follow_the_sampled_points_closed_form():
     assert np.abs(V.grid("tsdf")[both] - D.grid("tsdf")[both]).max() < 2e-3
 
 
+@pytest.mark.parametrize("pose", ["identity", "x90", "oblique"])
+def test_scalable_activation_of_non_finite_huge_and_boundary_points(pose):
+    """orc_scalable_integrate's activated units equal the NumPy restatement (tests/unit_activation_ref.py) for +-inf, NaN,
+    -0, negative, subnormal, 1e30 and FLT_MAX depths (+inf also on the principal point) and for points whose w -+ trunc
+    lands exactly on a unit face or one float32 step beside it; a non-finite world coordinate activates nothing"""
+    import unit_activation_ref as ref
+    rng = np.random.default_rng(len(pose))
+    vl, ur, trunc = 1.0 / 64, 8, 1.0 / 16                 # unit 1/8 m: every face below is exact in f64
+    dims, origin = (64, 64, 64), (-0.5, -0.5, -0.5)       # units -4 .. 3: global unit 0 inside the box
+    if pose == "identity":
+        R = np.eye(3)
+    elif pose == "x90":
+        R = np.array([[1.0, 0, 0], [0, 0, -1], [0, 1, 0]])
+    else:
+        q = rng.normal(size=4)
+        a, b, c, d = q / np.linalg.norm(q)
+        R = np.array([[a * a + b * b - c * c - d * d, 2 * (b * c - a * d), 2 * (b * d + a * c)],
+                      [2 * (b * c + a * d), a * a - b * b + c * c - d * d, 2 * (c * d - a * b)],
+                      [2 * (b * d - a * c), 2 * (c * d + a * b), a * a - b * b - c * c + d * d]])
+    E = np.eye(4)
+    E[:3, :3] = R.T
+    E[:3, 3] = -R.T @ (-0.75 * R[:, 2])                    # 0.75 m behind the box centre, looking at it
+    H = W = 16
+    Kc = (12.0, 12.0, 8.0, 8.0)                            # the principal point is a sampled pixel (stride 2)
+    vals = [np.nan, np.inf, -np.inf, -0.0, -0.25, 2.0 ** -149, 1e30, float(np.finfo(np.float32).max)]
+    frames = []
+    for k in range(3):
+        d = np.zeros((H, W), np.float32)
+        d[::2, ::2] = rng.choice(np.array(vals, np.float32), (H // 2, W // 2))
+        d[8, 8] = np.inf
+        frames.append(d)
+    # on the optical axis w = -0.75 + depth along the view direction: w -+ trunc on the faces -1/8, 0, 1/8
+    edges = sorted({np.float32(0.75 + f + s * trunc) for f in (-0.125, 0.0, 0.125) for s in (-1, 1)})
+    d = np.zeros((H, W), np.float32)
+    for n, z in enumerate(edges):
+        d[0, 2 * n:2 * n + 2] = np.inf
+        d[8, 8] = z
+        for v in (np.nextafter(z, np.float32(0)), z, np.nextafter(z, np.float32(9))):
+            e = d.copy()
+            e[8, 8] = v
+            frames.append(e)
+    non_finite = 0
+    for d in frames:
+        V = oracle.o3d.Volume(dims, vl, trunc, origin)
+        _, touched = V.integrate_scalable(d, Kc, E, unit_res=ur, stride=2, return_touched=True)
+        want = ref.unit_activation(d, Kc, E, dims, vl, trunc, origin, ur, 2)
+        assert np.array_equal(touched.astype(bool), want["touched"])
+        w, finite = ref.sampled_world_points(d, Kc, E, 2)
+        non_finite += int((~finite).sum())
+        if finite.sum() == 0:
+            assert not touched.any()
+    assert non_finite > 30
+    if pose != "oblique":
+        # +inf on the principal point gives NaN on every axis under a pose of exact zeros
+        w, finite = ref.sampled_world_points(frames[0], Kc, E, 2)
+        assert np.isnan(w).all(axis=1).any()
+
+
 def test_scalable_needs_whole_units_on_the_world_grid():
     V = oracle.o3d.Volume(72, 0.004, 0.02, origin=(-0.144,) * 3)
     with pytest.raises(ValueError):

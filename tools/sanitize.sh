@@ -2,7 +2,8 @@
 # compute-sanitizer over the hot path (run on a GPU box):  bash tools/sanitize.sh > gpurun_out/sanitizer.log
 # memcheck + racecheck + synccheck on smoke() (a4, K3 with named barriers / shared flag words / persistent
 # claims, K4 marching cubes, K1, K2), on a small sharded-layout / unit-activation / colour integration, on colour
-# integrations whose RGB batches end exactly where their allocations do, and on the image kernels at their edges.
+# integrations whose RGB batches end exactly where their allocations do, on unit activation with 8^3 units and two
+# mask words per row, and on the image kernels at their edges.
 set -u
 CS=/usr/local/cuda/bin/compute-sanitizer
 PY='
@@ -27,6 +28,10 @@ for kw in (dict(unit_activation=True), dict(gz0=8, z_total=64, z_interleave=2), 
         v.integrate_batch(d, col, sc["intrinsic"], sc["E"])
         if "gz0" not in kw:
             v.extract_triangle_mesh(); v.extract_point_cloud()
+# unit activation with 8^3 units and two mask words per (ux, uy) row (nuz = 64), stride 3
+v = DenseTSDFVolume(sc["voxel_length"], sc["sdf_trunc"], (64, 64, 512), org, color=False, device=dev, unit_activation=True,
+                    unit_resolution=8, depth_sampling_stride=3)
+v.integrate_batch(d, None, sc["intrinsic"], sc["E"])
 mdem.colorize(np.random.default_rng(0).uniform(0.1, 3, (120, 160)).astype(np.float32), cmap="viridis", invalid_val=0)
 # image kernels at their edges: a K1 batch of 65 images of 45 x 101 px (H*W = 1 mod 4: every image after the first
 # off a 16-byte boundary), a K2 call of 130 frames (three emit chunks of poses) and a K1f image holding NaN pixels
